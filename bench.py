@@ -2,6 +2,7 @@
 """bench.py -- pairwise OT distances / second on the PILOT patient-distance hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c5] [--rows R]
+                    [--dump-outputs DIR]
 
 Default workload = the configuration BASELINE.json's metric is quoted on, configs[4] ("c5", the scaling
 sweep): 20 000 samples x 64 cell types, ALL pairs with BOTH solvers -- exact EMD (199 990 000 unordered
@@ -178,6 +179,28 @@ def c5_units(S, rows=None):
     return rows * (2 * S - rows - 1) // 2, rows * S
 
 
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir, arrays, rows=None):
+    """--dump-outputs: write each device array the timed path returned in its last step as out_dir/<name>.npy.
+    Together they take at most DUMP_BYTES: an array larger than its share is written as a fixed, seeded sample of
+    its rows (of its first `rows` rows, the band a --rows step computes), in increasing order, so that the files of
+    two builds run with the same arguments hold the same entries."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        n = a.shape[0] if rows is None else rows
+        row_bytes = a[0].numel() * a.element_size()
+        if n * row_bytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(n, share // row_bytes, replace=False))
+            a = a[torch.from_numpy(idx).to(a.device)]
+        else:
+            a = a[:n]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def run_reference_c5(args):
     """Reference arm: the reference's CPU path for the same job on the host cores, every step a bounded sample
     (n ordered EMD problems + n ordered Sinkhorn problems = the fraction n / S^2 of the job: the reference
@@ -274,6 +297,8 @@ def run_c5(args):
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"emd": dense_e, "sinkhorn": dense_s}, rows)
     t = torch.tensor([ms_total], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -601,6 +626,8 @@ def run_cells(args):
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pairs": dense, "proportions": props, "cost": cost})
     t = torch.tensor([ms_total], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -743,7 +770,14 @@ def main():
     ap.add_argument("--workload", default="c5", choices=["c1", "c2", "c3", "c4", "c5"])
     ap.add_argument("--rows", type=int, default=None,
                     help="c5 only: restrict a step to the first R rows of both matrices (default: all 20000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the matrices the last timed step computed to DIR/<name>.npy (float64, at most 60 MB "
+                         "in all: a larger matrix as a fixed, seeded sample of its rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 path computes; it does not apply to --impl reference")
     if args.impl == "reference":
         (run_reference_c5 if args.workload == "c5" else run_reference_cells)(args)
     elif args.workload == "c5":

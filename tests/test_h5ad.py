@@ -1,10 +1,10 @@
 """(f)-3 host ingest: the built-in .h5ad (HDF5) reader and the real-data golden fixture.
 
-The reader is checked on the two real HDF5 files this image holds: the reference's tutorial data set (old-style
-groups, contiguous datasets, variable-length strings in global heaps, categorical columns, attributes) and SciPy's
-MATLAB-7.3 test file (512-byte user block, version-2 layout message; content known from SciPy's own test).  Chunked,
-shuffled and deflated datasets come from a minimal writer of our own (tests/h5_writer.py): no HDF5 library exists
-here to write them.  Sparse X and version-2 object headers are implemented from the format specification only."""
+The reader is checked on two real HDF5 files: the reference's tutorial data set (old-style groups, contiguous datasets,
+variable-length strings in global heaps, categorical columns, attributes; only where a PILOT checkout is mounted) and
+SciPy's MATLAB-7.3 test file (a copy in tests/golden; 512-byte user block, version-2 layout message; content known from
+SciPy's own test).  Chunked, shuffled and deflated datasets come from a minimal writer of our own
+(tests/h5_writer.py), so the tests need no HDF5 library.  Sparse X and version-2 object headers are implemented from the format specification only."""
 import os
 
 import numpy as np
@@ -78,10 +78,8 @@ def test_oracle_restatement_on_the_real_data_fixture():
 
 
 def test_matlab73_file_of_scipy():
-    import scipy.io
-    path = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if not os.path.isfile(path):
-        pytest.skip("SciPy test data not installed")
+    # a copy of SciPy's scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat (BSD-3-Clause)
+    path = os.path.join(os.path.dirname(GOLDEN), "testhdf5_7.4_GLNX86.mat")
     f = h5ad.H5File(path)                       # HDF5 behind a 512-byte user block
     assert f.root.keys() == ["testdouble"]
     np.testing.assert_allclose(f["testdouble"].read().ravel(), np.linspace(0, 2 * np.pi, 9), rtol=1e-15)
