@@ -1,29 +1,49 @@
 // C-ABI entry of kernel (3): dispatch between the batched shared-Gibbs-kernel solver and
 // the reference-form kernel (reference call site: pilotpy/tools/Trajectory.py:513-515).
+#include <stdint.h>
 #include <stdlib.h>
 #include "sinkhorn.cuh"
 
 namespace pilot {
 
-struct SkWs {
-    unsigned long long *counter_fast, *n_redo, *counter_slow;
-    double *setup, *scratch;
-    long long *redo;
+// the device counters in the workspace's 256-byte header, zeroed at the start of every call
+struct SkCounters {
+    unsigned long long fast;    // next problem of the warp-form, panel and FP32 kernels
+    unsigned long long n_redo;  // problems queued for the reference-form kernel
+    unsigned long long slow;    // next work item of the reference-form kernel
+    unsigned long long n_tail;  // problems the panels handed over
+    unsigned long long tail;    // next handed-over problem of the tail kernel
 };
 
-// every slot of the panel kernel could in principle be handed over to the tail kernel
-static size_t sk_tail_slots() { return (size_t)sm_count() * skb_slots_per_cta(); }
-static size_t sk_tail_rec_bytes() { return (sk_tail_slots() * sizeof(SkTailRec) + 255) / 256 * 256; }
-static size_t sk_tail_uv_bytes(int KP) { return sk_tail_slots() * 2 * KP * sizeof(double); }
+// the regions of a call's workspace
+struct SkWorkspace {
+    SkCounters *ctr;
+    double *setup, *scratch;
+    long long *redo;
+    SkTailRec *tail_rec;
+    double *tail_uv;
+    size_t bytes;  // end of the last region
+};
 
-static size_t sk_ws_bytes(int K)
+// carves the workspace at `base` (nullptr: only its size)
+static SkWorkspace sk_workspace(void *base, int K)
 {
     const int KP = skb_pad(K <= 64 ? K : 64);
-    return 256 + skb_setup_bytes(KP) + skb_scratch_bytes(KP, sm_count()) + (size_t)SK_REDO_CAP * sizeof(long long) +
-           sk_tail_rec_bytes() + sk_tail_uv_bytes(KP);
+    const size_t tail_slots = (size_t)sm_count() * skb_slots_per_cta();  // every panel slot could be handed over
+    uintptr_t p = (uintptr_t)base;
+    const auto take = [&p](size_t bytes) { const uintptr_t r = p; p += bytes; return r; };
+    SkWorkspace ws;
+    ws.ctr = (SkCounters *)take(256);
+    ws.setup = (double *)take(skb_setup_bytes(KP));
+    ws.scratch = (double *)take(skb_scratch_bytes(KP, sm_count()));
+    ws.redo = (long long *)take((size_t)SK_REDO_CAP * sizeof(long long));
+    ws.tail_rec = (SkTailRec *)take((tail_slots * sizeof(SkTailRec) + 255) / 256 * 256);
+    ws.tail_uv = (double *)take(tail_slots * 2 * KP * sizeof(double));
+    ws.bytes = p - (uintptr_t)base;
+    return ws;
 }
 
-size_t sinkhorn_ws_bytes(int K) { return sk_ws_bytes(K); }
+size_t sinkhorn_ws_bytes(int K) { return sk_workspace(nullptr, K).bytes; }
 
 }  // namespace pilot
 
@@ -42,26 +62,19 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     PILOT_CHECK_ARG(algo == 0 || algo == 1 || algo == 3, "pilot_sinkhorn_pairs: algo %d", algo);
     PILOT_CHECK_ARG(precision == PILOT_F64 || precision == PILOT_F32, "pilot_sinkhorn_pairs: precision=%d", precision);
     PILOT_CHECK_ARG(sinkhorn_ref_smem(K) <= 200 * 1024, "pilot_sinkhorn_pairs: K=%d too large (max ~150)", K);
-    PILOT_CHECK_ARG(workspace_bytes >= sk_ws_bytes(K), "pilot_sinkhorn_pairs: workspace %zu < %zu bytes",
-                    workspace_bytes, sk_ws_bytes(K));
+    const SkWorkspace ws = sk_workspace(workspace, K);
+    PILOT_CHECK_ARG(workspace_bytes >= ws.bytes, "pilot_sinkhorn_pairs: workspace %zu < %zu bytes", workspace_bytes,
+                    ws.bytes);
     PairMap pm;
     int rc = make_pair_map(range, S, &pm);
     if (rc) return rc;
     if (pm.n_local == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     SkParams prm{reg, stop_thr, tau, num_iter_max, check_every};
+    const SkOut res{out, iters, absorptions, status, ws.redo, &ws.ctr->n_redo};
 
-    unsigned char *p = (unsigned char *)workspace;
-    SkWs ws;
-    ws.counter_fast = (unsigned long long *)p;
-    ws.n_redo = ws.counter_fast + 1;
-    ws.counter_slow = ws.counter_fast + 2;
-    PILOT_CUDA(cudaMemsetAsync(p, 0, 256, st));
-    if (algo == 1 || K > 64)
-        return sinkhorn_ref_launch(props, K, cost, prm, pm, nullptr, nullptr, 0, out, iters, absorptions, status,
-                                   ws.counter_slow, st);
-    const int KP = skb_pad(K);
-    ws.redo = (long long *)(p + 256 + skb_setup_bytes(KP) + skb_scratch_bytes(KP, sm_count()));
+    PILOT_CUDA(cudaMemsetAsync(ws.ctr, 0, sizeof(SkCounters), st));
+    if (algo == 1 || K > 64) return sinkhorn_ref_launch(props, K, cost, prm, pm, res, SK_SOLVE_ALL, &ws.ctr->slow, st);
     long long redo_cap = SK_REDO_CAP;
     // (PILOT_SK_REDO_CAP, tests only: a smaller list capacity, to exercise the overflow scan)
     if (const char *e = getenv("PILOT_SK_REDO_CAP")) {
@@ -71,21 +84,12 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     if (precision == PILOT_F32) {
         // single precision: per-problem kernel in registers (sinkhorn_f32.cu); what it cannot carry (NaN/Inf,
         // zero masses) goes to the FP64 reference-form kernel like in the FP64 mode
-        rc = skf_launch(props, K, cost, prm, pm, out, iters, absorptions, status, ws.counter_fast, ws.redo,
-                        ws.n_redo, st);
+        rc = skf_launch(props, K, cost, prm, pm, res, &ws.ctr->fast, st);
         if (rc) return rc;
-        return sinkhorn_ref_launch(props, K, cost, prm, pm, ws.redo, ws.n_redo, redo_cap, out, iters, absorptions,
-                                   status, ws.counter_slow, st);
+        return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, st);
     }
-    ws.setup = (double *)(p + 256);
-    ws.scratch = (double *)(p + 256 + skb_setup_bytes(KP));
-    unsigned char *ptail = (unsigned char *)ws.redo + (size_t)SK_REDO_CAP * sizeof(long long);
-    SkTail tail;
-    tail.rec = (SkTailRec *)ptail;
-    tail.uv = (double *)(ptail + sk_tail_rec_bytes());
-    tail.n_tail = ws.counter_fast + 3;
-    tail.evict_max = 2;  // measured: 0 (no hand-over) 2.23 ms, 2: 1.45 ms, 4: 1.44 ms, 7: 1.56 ms for 10^4 problems at K = 64
-    unsigned long long *tail_counter = ws.counter_fast + 4;
+    // evict_max measured: 0 (no hand-over) 2.23 ms, 2: 1.45 ms, 4: 1.44 ms, 7: 1.56 ms for 10^4 problems at K = 64
+    const SkTail tail{ws.tail_rec, ws.tail_uv, &ws.ctr->n_tail, 2};
     rc = skb_setup(cost, K, prm, ws.setup, st);
     if (rc) return rc;
     // The cost is symmetric in PILOT (a pdist matrix) but the API takes any matrix.  Whether it is is known
@@ -103,8 +107,7 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     // solved by the same arithmetic however the pair space is partitioned: results are partition-invariant bit for bit.
     const bool warp_form = algo == 0 && K <= swk_max_k() && (K > 16 || (long long)S * S < 200000);
     if (warp_form) {  // symmetric cost only; an asymmetric one falls through to the general panels below
-        rc = swk_launch(props, K, prm, pm, ws.setup, out, iters, absorptions, status, ws.counter_fast, ws.redo,
-                        ws.n_redo, st);
+        rc = swk_launch(props, K, prm, pm, ws.setup, res, &ws.ctr->fast, st);
         if (rc) return rc;
     }
     const long long spw = skb_slots_per_warp();
@@ -115,17 +118,14 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     if (warp_cap < 1) warp_cap = 1;
     for (int sym = warp_form ? 0 : 1; sym >= 0; --sym) {
         rc = skb_launch(props, K, prm, pm, ws.setup, ws.scratch, (int)ctas, slot_cap, (int)warp_cap, sym != 0,
-                        tail, out, iters, absorptions, status, ws.counter_fast, ws.redo, ws.n_redo, st);
+                        tail, res, &ws.ctr->fast, st);
         if (rc) return rc;
     }
     // the stragglers the panels handed over continue in warp form
     for (int sym = warp_form ? 0 : 1; sym >= 0; --sym) {
-        rc = skt_launch(props, K, prm, pm, ws.setup, ws.scratch, sym != 0, tail, tail_counter, out, iters,
-                        absorptions, status, ws.redo, ws.n_redo, st);
+        rc = skt_launch(props, K, prm, pm, ws.setup, ws.scratch, sym != 0, tail, &ws.ctr->tail, res, st);
         if (rc) return rc;
     }
-    if (rc) return rc;
     // problems the scaled form could not represent (normally none): reference-form kernel
-    return sinkhorn_ref_launch(props, K, cost, prm, pm, ws.redo, ws.n_redo, redo_cap, out, iters, absorptions,
-                               status, ws.counter_slow, st);
+    return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, st);
 }

@@ -77,23 +77,6 @@ __device__ __forceinline__ void dmma884(double &c0, double &c1, double a, double
                  : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-// branch-free x / y for finite positive y.  FP64-pipe instructions are what the element-wise phases
-// pay for (they queue behind the DMMAs): 4 here.
-__device__ __forceinline__ double fast_div(double x, double y)
-{
-    // 20-bit seed r, e = 1 - y r, q = x r (1 + e + e^2): relative error e^3 ~ 2^-60 before the final
-    // rounding; 4 FP64-pipe instructions in a dependent chain of 3
-    double r;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
-    const double e = fma(-y, r, 1.0);
-    const double q0 = x * r;
-    return fma(q0, fma(e, e, e), q0);
-}
-
-// |x| as an ordered integer: for non-NaN doubles the bit pattern orders like the value, NaN / Inf
-// sort above every finite value -- max / threshold tests without touching the FP64 pipe
-__device__ __forceinline__ long long abs_bits(double x) { return __double_as_longlong(x) & 0x7fffffffffffffffLL; }
-
 // swizzled matrix addressing: column ^ 4 * (row % 4).  An A-fragment load reads rows 4*ks + t
 // (t = 0..3) at columns 8*m + g; 64-bit shared loads are served per half-warp (g = 0..3 / 4..7), and
 // with this swizzle the four rows of a half-warp fall into four different 8-bank groups: 2
@@ -106,16 +89,15 @@ __device__ __forceinline__ int swz(int row, int col) { return col ^ ((row & 3) <
 template <int KP, int KC, bool FULL, bool SYM>
 __global__ void __launch_bounds__(SKB_WARPS * 32, 1)
 sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, PairMap pm, int slot_cap, int warp_cap,
-                        const double *__restrict__ gK0, const double *__restrict__ gK0T,
-                        const double *__restrict__ gMK, const double *__restrict__ gc0,
-                        double *__restrict__ scratch,  // [gridDim * WARPS * 8][2][KP] rea / reb
-                        SkTail tail, double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
-                        int *__restrict__ status_out, unsigned long long *__restrict__ counter,
+                        SkSetup s, double *__restrict__ scratch,  // [gridDim * WARPS * 8][2][KP] rea / reb
+                        SkTail tail, unsigned long long *__restrict__ counter, double *__restrict__ out,
+                        int *__restrict__ iters_out, int *__restrict__ abs_out, int *__restrict__ status_out,
                         long long *__restrict__ redo_list, unsigned long long *__restrict__ n_redo)
 {
-    // the symmetric and the general variant are both enqueued; the flag the setup kernel left behind the
-    // c0 vector decides on the device which one runs (no host read-back in a Sinkhorn call)
-    if ((reinterpret_cast<const int *>(gc0 + KP)[0] != 0) == SYM) return;
+    const SkOut res{out, iters_out, abs_out, status_out, redo_list, n_redo};
+    // the symmetric and the general variant are both enqueued; the setup kernel's asymmetry flag decides on
+    // the device which one runs (no host read-back in a Sinkhorn call)
+    if ((*s.asym != 0) == SYM) return;
     constexpr int MT = KC / 8;   // accumulator row tiles
     constexpr int KS = KC / 4;   // k-steps of 4
     constexpr int PS = SKB_SPW;  // panel row stride (doubles): 64-byte rows, conflict-free as they are
@@ -137,11 +119,11 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
     double *sB = sA + SKB_SPW * KP;
     for (int e = threadIdx.x; e < KP * KP; e += blockDim.x) {
         const int r = e / KP, c = e - r * KP;
-        sK0[r * KP + swz(r, c)] = gK0[e];
-        if (sym) sSecond[e] = gMK[e];                    // plain [i][j]
-        else sSecond[r * KP + swz(r, c)] = gK0T[e];
+        sK0[r * KP + swz(r, c)] = s.K0[e];
+        if (sym) sSecond[e] = s.MK[e];                   // plain [i][j]
+        else sSecond[r * KP + swz(r, c)] = s.K0T[e];
     }
-    for (int e = threadIdx.x; e < KP; e += blockDim.x) sc0[e] = gc0[e];
+    for (int e = threadIdx.x; e < KP; e += blockDim.x) sc0[e] = s.c0[e];
     __syncthreads();
     if (warp >= warp_cap) return;  // small batches: fewer warps per scheduler = shorter iteration latency
 
@@ -259,7 +241,7 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                 double cost = 0.0;
                 if (stt >= 0) {
                     // cost = sum_j Vt_j * sum_i (M o K0)_ij Ut_i ; lane = column j
-                    const double *mk = sym ? sSecond : gMK;
+                    const double *mk = sym ? sSecond : s.MK;
                     for (int j = lane; j < KC; j += 32) {  // panel rows >= KC are never written
                         double w0 = 0.0, w1 = 0.0;
                         for (int i = 0; i + 1 < K; i += 2) {
@@ -276,19 +258,7 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                 w = __shfl_sync(0xffffffffu, w, 0);
                 const bool mine = t == tt;
                 __syncwarp();  // every lane has read the slot's U, V columns before its owners refill them
-                if (mine && g == 0) {
-                    if (stt >= 0) {
-                        out[sl[h]] = cost;
-                        if (iters_out) iters_out[sl[h]] = s_ii[h];
-                        if (abs_out) abs_out[sl[h]] = s_abs[h];
-                        if (status_out) status_out[sl[h]] = stt;
-                    } else {
-                        const unsigned long long slot = atomicAdd(n_redo, 1ULL);
-                        if ((long long)slot < SK_REDO_CAP) redo_list[slot] = sl[h];
-                        out[sl[h]] = __longlong_as_double(SK_REDO_MARK);
-                        if (status_out) status_out[sl[h]] = -1;
-                    }
-                }
+                if (mine && g == 0) sk_store(res, sl[h], stt, cost, s_ii[h], s_abs[h]);
                 if (mine) {
                     SKB_ASSIGN(h, w);
 #pragma unroll
@@ -347,9 +317,9 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                     for (int h = 0; h < 2; ++h)
                         if (s_act[h]) {
                             const double tv = s_fresh[h] ? sc0[row] : acc[m][h];
-                            vv[h] = fast_div(num[m][h], tv);
+                            vv[h] = sk_div(num[m][h], tv);
                             const double uu = s_hasabs[h] ? vv[h] * rea0[(2 * h + 1) * KP + row] : vv[h];
-                            mxv[h] = max(mxv[h], abs_bits(uu));
+                            mxv[h] = max(mxv[h], sk_abs_bits(uu));
                         }
                 }
                 *reinterpret_cast<double2 *>(Vc + 8 * m * PS) = make_double2(vv[0], vv[1]);
@@ -385,9 +355,9 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                     const int row = 8 * m + g;
                     un[m][h] = 0.0;
                     if (s_act[h] && ROW_OK(row)) {
-                        un[m][h] = fast_div(num[m][h], acc[m][h]);
+                        un[m][h] = sk_div(num[m][h], acc[m][h]);
                         const double uu = s_hasabs[h] ? un[m][h] * rea0[(2 * h) * KP + row] : un[m][h];
-                        mxu[h] = max(mxu[h], abs_bits(uu));
+                        mxu[h] = max(mxu[h], sk_abs_bits(uu));
                     }
                 }
             bool absorb[2];
@@ -396,7 +366,7 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                 long long mx = max(mxu[h], mxv[h]);
 #pragma unroll
                 for (int o = 4; o < 32; o <<= 1) mx = max(mx, __shfl_xor_sync(gmask, mx, o));
-                const bool bad = mx >= 0x7ff0000000000000LL;  // NaN or Inf anywhere in u, v
+                const bool bad = mx >= SK_NONFINITE_BITS;  // NaN or Inf anywhere in u, v
                 absorb[h] = s_act[h] && !bad && mx > __double_as_longlong(prm.tau);
                 if (s_act[h]) {
                     s_bad[h] = bad;
@@ -420,7 +390,8 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
                                 double &vref = h ? vo.y : vo.x;
                                 rea0[(2 * h) * KP + row] = 1.0 / un[m][h];
                                 rea0[(2 * h + 1) * KP + row] = 1.0 / vref;
-                                // keep e^{+-alpha/reg} comfortably inside the FP64 range
+                                // keep e^{+-alpha/reg} comfortably inside the FP64 range (spelled out here: through
+                                // sk_out_of_range the KP = 48, 64 panels take a register or spill more)
                                 rb[h] |= !(un[m][h] > 1e-250 && un[m][h] < 1e250 && vref > 1e-250 && vref < 1e250);
                                 un[m][h] *= invK;
                                 vref *= invK;
@@ -451,6 +422,12 @@ sinkhorn_batched_kernel(const double *__restrict__ props, int K, SkParams prm, P
 }
 
 size_t skb_setup_bytes(int KP) { return sizeof(double) * ((size_t)3 * KP * KP + KP + 32); }
+// the flag is an int in the room behind c0
+SkSetup sk_setup_view(const double *setup, int KP)
+{
+    const size_t n = (size_t)KP * KP;
+    return {setup, setup + n, setup + 2 * n, setup + 3 * n, reinterpret_cast<const int *>(setup + 3 * n + KP)};
+}
 size_t skb_smem_bytes(int KP)
 {
     const size_t stage = KP <= 32 ? (size_t)SKB_WARPS * 2 * SKB_SPW * KP : 0;  // a, b of every slot
@@ -468,57 +445,44 @@ int skb_warps() { return SKB_WARPS; }
 
 template <int KP, int KC, bool FULL, bool SYM>
 static int skb_launch_t(const double *props, int K, const SkParams &prm, const PairMap &pm, int slot_cap, int warp_cap,
-                        const double *setup, double *scratch, const SkTail &tail, int ctas, double *out, int *iters, int *absn,
-                        int *status, unsigned long long *counter, long long *redo, unsigned long long *n_redo,
-                        cudaStream_t st)
+                        const SkSetup &s, double *scratch, const SkTail &tail, int ctas, const SkOut &res,
+                        unsigned long long *counter, cudaStream_t st)
 {
     const size_t smem = skb_smem_bytes(KP);
     PILOT_CUDA(cudaFuncSetAttribute(sinkhorn_batched_kernel<KP, KC, FULL, SYM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)smem));
-    const double *K0 = setup, *K0T = K0 + KP * KP, *MK = K0T + KP * KP, *c0 = MK + KP * KP;
     sinkhorn_batched_kernel<KP, KC, FULL, SYM><<<ctas, SKB_WARPS * 32, smem, st>>>(
-        props, K, prm, pm, slot_cap, warp_cap, K0, K0T, MK, c0, scratch, tail, out, iters, absn, status, counter, redo,
-        n_redo);
+        props, K, prm, pm, slot_cap, warp_cap, s, scratch, tail, counter, res.out, res.iters, res.absn, res.status,
+        res.redo, res.n_redo);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
 
-// computes K0, K0^T, M o K0, c0 and the asymmetry flag (an int behind c0: != 0 when M differs from its
-// transpose); the solver kernels read the flag themselves
+// fills the buffer sk_setup_view describes
 int skb_setup(const double *cost, int K, const SkParams &prm, double *setup, cudaStream_t st)
 {
     const int KP = skb_pad(K);
-    PILOT_CUDA(cudaMemsetAsync(setup + 3 * KP * KP + KP, 0, sizeof(double), st));
-    skb_setup_kernel<<<8, 256, 0, st>>>(cost, K, KP, prm.reg, setup, setup + KP * KP, setup + 2 * KP * KP,
-                                        setup + 3 * KP * KP, reinterpret_cast<int *>(setup + 3 * KP * KP + KP));
+    const SkSetup s = sk_setup_view(setup, KP);
+    int *asym = const_cast<int *>(s.asym);
+    PILOT_CUDA(cudaMemsetAsync(asym, 0, sizeof(int), st));
+    skb_setup_kernel<<<8, 256, 0, st>>>(cost, K, KP, prm.reg, setup, const_cast<double *>(s.K0T),
+                                        const_cast<double *>(s.MK), const_cast<double *>(s.c0), asym);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
 
 // `setup` must already hold the output of skb_setup
-int skb_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, double *setup, double *scratch,
-               int ctas, int slot_cap, int warp_cap, bool symmetric, const SkTail &tail, double *out, int *iters,
-               int *absn, int *status, unsigned long long *counter, long long *redo, unsigned long long *n_redo,
-               cudaStream_t st)
+int skb_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
+               double *scratch, int ctas, int slot_cap, int warp_cap, bool symmetric, const SkTail &tail,
+               const SkOut &res, unsigned long long *counter, cudaStream_t st)
 {
     const int KP = skb_pad(K);
-    const int h_asym = symmetric ? 0 : 1;
+    const SkSetup s = sk_setup_view(setup, KP);
+    // FULL: K fills the compute extent KC, no row masks
 #define SKB_GO(KPV, KCV)                                                                                          \
-    do {                                                                                                          \
-        if (h_asym == 0) {                                                                                        \
-            if (K == KCV)                                                                                         \
-                return skb_launch_t<KPV, KCV, true, true>(props, K, prm, pm, slot_cap, warp_cap, setup, scratch,   \
-                                                          tail, ctas, out, iters, absn, status, counter, redo,     \
-                                                          n_redo, st);                                             \
-            return skb_launch_t<KPV, KCV, false, true>(props, K, prm, pm, slot_cap, warp_cap, setup, scratch, tail, \
-                                                       ctas, out, iters, absn, status, counter, redo, n_redo, st); \
-        }                                                                                                         \
-        if (K == KCV)                                                                                             \
-            return skb_launch_t<KPV, KCV, true, false>(props, K, prm, pm, slot_cap, warp_cap, setup, scratch, tail, \
-                                                       ctas, out, iters, absn, status, counter, redo, n_redo, st); \
-        return skb_launch_t<KPV, KCV, false, false>(props, K, prm, pm, slot_cap, warp_cap, setup, scratch, tail,   \
-                                                    ctas, out, iters, absn, status, counter, redo, n_redo, st);    \
-    } while (0)
+    return (symmetric ? (K == KCV ? skb_launch_t<KPV, KCV, true, true> : skb_launch_t<KPV, KCV, false, true>)     \
+                      : (K == KCV ? skb_launch_t<KPV, KCV, true, false> : skb_launch_t<KPV, KCV, false, false>))( \
+        props, K, prm, pm, slot_cap, warp_cap, s, scratch, tail, ctas, res, counter, st)
     if (KP == 16) SKB_GO(16, 16);
     if (KP == 32) { if (K <= 24) SKB_GO(32, 24); SKB_GO(32, 32); }
     if (KP == 48) { if (K <= 40) SKB_GO(48, 40); SKB_GO(48, 48); }

@@ -65,10 +65,11 @@ __device__ __forceinline__ float fdiv_fast(float x, float y)
 template <int KP>
 __global__ void __launch_bounds__(SKF_WARPS * 32, 1)
 sinkhorn_f32_kernel(const double *__restrict__ props, int K, const double *__restrict__ M, SkParams prm, PairMap pm,
-                    double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
-                    int *__restrict__ status_out, unsigned long long *__restrict__ counter,
-                    long long *__restrict__ redo_list, unsigned long long *__restrict__ n_redo)
+                    unsigned long long *__restrict__ counter, double *__restrict__ out, int *__restrict__ iters_out,
+                    int *__restrict__ abs_out, int *__restrict__ status_out, long long *__restrict__ redo_list,
+                    unsigned long long *__restrict__ n_redo)
 {
+    const SkOut res{out, iters_out, abs_out, status_out, redo_list, n_redo};
     using S = SkfShape<KP>;
     constexpr int TR = S::TR, TC = S::TC, NV = S::NV;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -230,13 +231,13 @@ sinkhorn_f32_kernel(const double *__restrict__ props, int K, const double *__res
             }
         }
 
+        float acc = 0.0f;
         if (status >= 0) {
             // cost = sum_ij M_ij u_i K_ij v_j with the state at the stop (su holds u, v is current)
             __syncwarp();
 #pragma unroll
             for (int e = 0; e < NV; ++e) sv[col0 + e] = v[e];
             __syncwarp();
-            float acc = 0.0f;
 #pragma unroll
             for (int i = 0; i < TR; ++i) {
                 const int gi = trow + i;
@@ -250,45 +251,33 @@ sinkhorn_f32_kernel(const double *__restrict__ props, int K, const double *__res
             }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(SKF_FULL, acc, o);
-            if (lane == 0) {
-                out[w] = (double)(acc * unscale);
-                if (iters_out) iters_out[w] = ii;
-                if (abs_out) abs_out[w] = nabs;
-                if (status_out) status_out[w] = status;
-            }
-        } else if (lane == 0) {
-            const unsigned long long slot = atomicAdd(n_redo, 1ULL);
-            if ((long long)slot < SK_REDO_CAP) redo_list[slot] = (long long)w;
-            out[w] = __longlong_as_double(SK_REDO_MARK);
-            if (status_out) status_out[w] = -1;
         }
+        if (lane == 0) sk_store(res, (long long)w, status, (double)(acc * unscale), ii, nabs);
         __syncwarp();
     }
 }
 
 template <int KP>
 static int skf_launch_t(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
-                        double *out, int *iters, int *absn, int *status, unsigned long long *counter,
-                        long long *redo, unsigned long long *n_redo, cudaStream_t st)
+                        const SkOut &res, unsigned long long *counter, cudaStream_t st)
 {
     const size_t smem = sizeof(float) * ((size_t)2 * KP * KP + (size_t)SKF_WARPS * 4 * KP);
     PILOT_CUDA(cudaFuncSetAttribute(sinkhorn_f32_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     long long ctas = (pm.n_local + SKF_WARPS - 1) / SKF_WARPS;
     if (ctas > sm_count()) ctas = sm_count();
     if (ctas < 1) ctas = 1;
-    sinkhorn_f32_kernel<KP><<<(unsigned)ctas, SKF_WARPS * 32, smem, st>>>(props, K, cost, prm, pm, out, iters, absn,
-                                                                         status, counter, redo, n_redo);
+    sinkhorn_f32_kernel<KP><<<(unsigned)ctas, SKF_WARPS * 32, smem, st>>>(props, K, cost, prm, pm, counter, res.out,
+                                                                         res.iters, res.absn, res.status, res.redo,
+                                                                         res.n_redo);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
 
-int skf_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm, double *out,
-               int *iters, int *absn, int *status, unsigned long long *counter, long long *redo,
-               unsigned long long *n_redo, cudaStream_t st)
+int skf_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
+               const SkOut &res, unsigned long long *counter, cudaStream_t st)
 {
-    if (K <= 32)
-        return skf_launch_t<32>(props, K, cost, prm, pm, out, iters, absn, status, counter, redo, n_redo, st);
-    return skf_launch_t<64>(props, K, cost, prm, pm, out, iters, absn, status, counter, redo, n_redo, st);
+    if (K <= 32) return skf_launch_t<32>(props, K, cost, prm, pm, res, counter, st);
+    return skf_launch_t<64>(props, K, cost, prm, pm, res, counter, st);
 }
 
 }  // namespace pilot

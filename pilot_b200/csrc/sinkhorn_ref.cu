@@ -41,7 +41,7 @@ __device__ __forceinline__ double block_sum64(double v, double *red)
     return r;
 }
 
-// mode 0: every local problem; mode 1: the problems of `list` (at most max_list of them); mode 2: only if
+// mode 0: every local problem; mode 1: the problems of the redo list (at most max_list of them); mode 2: only if
 // more than max_list problems were queued (the list overflowed): scan out[] for the redo marker the fast
 // kernels left behind and solve those (the listed ones were overwritten by mode 1 already).
 __global__ void __launch_bounds__(SKR_MAX_WARPS * 32)
@@ -202,12 +202,11 @@ size_t sinkhorn_ref_smem(int K)
 }
 
 int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
-                        const long long *list, const unsigned long long *n_list_dev, long long max_list,
-                        double *out, int *iters, int *absorptions, int *status, unsigned long long *counter,
-                        cudaStream_t st)
+                        const SkOut &res, long long redo_cap, unsigned long long *counter, cudaStream_t st)
 {
+    const bool queued = redo_cap != SK_SOLVE_ALL;
     // with a device-side list the amount of work is unknown here: launch one wave and let the CTAs loop
-    const long long n_work = list ? (long long)sm_count() * 4 : pm.n_local;
+    const long long n_work = queued ? (long long)sm_count() * 4 : pm.n_local;
     if (n_work <= 0) return 0;
     const size_t smem = sinkhorn_ref_smem(K);
     const int threads = skr_threads(K);
@@ -219,10 +218,11 @@ int sinkhorn_ref_launch(const double *props, int K, const double *cost, const Sk
     long long ctas = (long long)sm_count() * per_sm;
     if (ctas > n_work) ctas = n_work;
     // modes 1 and 2 run back to back on the stream and share the counter: reset it before each
-    for (int mode = list ? 1 : 0; mode <= (list ? 2 : 0); ++mode) {
+    for (int mode = queued ? 1 : 0; mode <= (queued ? 2 : 0); ++mode) {
         PILOT_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-        sinkhorn_ref_kernel<<<(unsigned)ctas, threads, smem, st>>>(props, K, cost, prm, pm, mode, list, n_list_dev,
-                                                                  max_list, out, iters, absorptions, status, counter);
+        sinkhorn_ref_kernel<<<(unsigned)ctas, threads, smem, st>>>(props, K, cost, prm, pm, mode, res.redo, res.n_redo,
+                                                                  redo_cap, res.out, res.iters, res.absn, res.status,
+                                                                  counter);
         PILOT_LAUNCH_CHECK();
     }
     return 0;

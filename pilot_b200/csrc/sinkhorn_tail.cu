@@ -23,17 +23,6 @@ namespace pilot {
 
 constexpr int SKT_WARPS = 16;
 
-__device__ __forceinline__ double skt_div(double x, double y)
-{
-    // 20-bit seed r, e = 1 - y r, q = x r (1 + e + e^2): relative error e^3 ~ 2^-60 before the final
-    // rounding; 4 FP64-pipe instructions in a dependent chain of 3
-    double r;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
-    const double e = fma(-y, r, 1.0);
-    const double q0 = x * r;
-    return fma(q0, fma(e, e, e), q0);
-}
-
 // res[rr] = sum_i mat[i][row0 + rr] * buf[i] as ONE fma chain in ascending i per row -- the order in which the
 // DMMA panels accumulate (see the header) -- (mat is [KP][KP], i-major; the lane's R rows are adjacent, so
 // R = 2 reads them with one 128-bit load; buf is broadcast as 128-bit loads)
@@ -64,19 +53,15 @@ __device__ __forceinline__ void skt_matvec(const double *__restrict__ mat, int r
     for (int rr = 0; rr < R; ++rr) res[rr] = s[rr];
 }
 
-enum { SKT_PEND = 1, SKT_FORCE = 2, SKT_BAD = 4 };
-
 template <int KP, bool SYM>
 __global__ void __launch_bounds__(SKT_WARPS * 32, 1)
-sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, PairMap pm,
-                     const double *__restrict__ gK0, const double *__restrict__ gK0T,
-                     const double *__restrict__ gMK, const double *__restrict__ gc0,
-                     const int *__restrict__ asym_flag,
-                     const double *__restrict__ scratch, SkTail tail,
-                     unsigned long long *__restrict__ tail_counter, double *__restrict__ out,
-                     int *__restrict__ iters_out, int *__restrict__ abs_out, int *__restrict__ status_out,
-                     long long *__restrict__ redo_list, unsigned long long *__restrict__ n_redo)
+sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, PairMap pm, SkSetup s,
+                     const double *__restrict__ scratch, SkTail tail, unsigned long long *__restrict__ tail_counter,
+                     double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
+                     int *__restrict__ status_out, long long *__restrict__ redo_list,
+                     unsigned long long *__restrict__ n_redo)
 {
+    const SkOut res{out, iters_out, abs_out, status_out, redo_list, n_redo};
     constexpr int R = (KP + 31) / 32;  // rows per lane
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double *sK0 = reinterpret_cast<double *>(smem_raw);  // [i][j]: column access for T = K0^T ut
@@ -84,11 +69,11 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
     double *sK0T = SYM ? sK0 : sMK + KP * KP;            // [j][i]: column access for S = K0 vt
     double *sbuf = (SYM ? sMK : sK0T) + KP * KP;         // per warp: broadcast copies of ut, vt
     const unsigned long long n_tail = *tail.n_tail;
-    if (n_tail == 0 || (*asym_flag != 0) == SYM) return;
+    if (n_tail == 0 || (*s.asym != 0) == SYM) return;
     for (int e = threadIdx.x; e < KP * KP; e += blockDim.x) {
-        sK0[e] = gK0[e];
-        sMK[e] = gMK[e];
-        if (!SYM) sK0T[e] = gK0T[e];
+        sK0[e] = s.K0[e];
+        sMK[e] = s.MK[e];
+        if (!SYM) sK0T[e] = s.K0T[e];
     }
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -103,7 +88,7 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
         row_ok[rr] = r < K;
         row[rr] = in_pad[rr] ? r : 0;
     }
-    const unsigned long long tau_bits = (unsigned long long)__double_as_longlong(prm.tau);
+    const long long tau_bits = __double_as_longlong(prm.tau);
     const double invK = 1.0 / K;
 
     for (;;) {
@@ -142,12 +127,12 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
                 // a slot can be handed over right after it was refilled: the panels take the first product
                 // K0^T (1/K) from the setup kernel's c0 (summed in another order), and so must we
 #pragma unroll
-                for (int rr = 0; rr < R; ++rr) T[rr] = __ldg(gc0 + row[rr]);
+                for (int rr = 0; rr < R; ++rr) T[rr] = __ldg(s.c0 + row[rr]);
             }
             if (ctl) {
-                if (ctl & SKT_BAD) { status = -1; break; }
+                if (ctl & SK_BAD) { status = -1; break; }
                 bool conv = false;
-                if (ctl & SKT_PEND) {
+                if (ctl & SK_PEND) {
                     // || vt o T - b ||^2 summed like the panels do: lane g takes rows g, 8 + g, ... in ascending
                     // order, then the butterfly over g
 #pragma unroll
@@ -164,34 +149,29 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
                     __syncwarp();
                 }
                 if (conv) { status = PILOT_ST_CONVERGED; break; }
-                if (ctl & SKT_FORCE) { status = PILOT_ST_MAXITER; break; }
+                if (ctl & SK_FORCE) { status = PILOT_ST_MAXITER; break; }
             }
             // ---- vt = b / T ----
 #pragma unroll
             for (int rr = 0; rr < R; ++rr) {
-                v[rr] = row_ok[rr] ? skt_div(b[rr], T[rr]) : 0.0;
+                v[rr] = row_ok[rr] ? sk_div(b[rr], T[rr]) : 0.0;
                 if (in_pad[rr]) vb[row[rr]] = v[rr];
             }
             __syncwarp();
             // ---- ut = a / (K0 vt) ----
             double S[R];
             skt_matvec<KP, R>(sK0T, row[0], vb, S);
-            unsigned long long mx = 0;
+            long long mx = 0;
 #pragma unroll
             for (int rr = 0; rr < R; ++rr) {
-                u[rr] = row_ok[rr] ? skt_div(a[rr], S[rr]) : 0.0;
-                // u, v of the reference = ut * rea, vt * reb; NaN / Inf sort above every finite value
-                const unsigned long long bu = (unsigned long long)__double_as_longlong(u[rr] * rea[rr]);
-                const unsigned long long bv = (unsigned long long)__double_as_longlong(v[rr] * reb[rr]);
-                mx = max(mx, max(bu, bv));
+                u[rr] = row_ok[rr] ? sk_div(a[rr], S[rr]) : 0.0;
+                // u, v of the reference = ut * rea, vt * reb
+                mx = max(mx, max(sk_abs_bits(u[rr] * rea[rr]), sk_abs_bits(v[rr] * reb[rr])));
             }
-            ctl = (until_check == 0) ? SKT_PEND : 0;
-            until_check = (until_check == 0 ? prm.check_every : until_check) - 1;
-            ++ii;
-            if (ii >= prm.num_iter_max) ctl |= SKT_FORCE;
+            ctl = sk_step(prm, until_check, ii);
             if (__any_sync(0xffffffffu, mx > tau_bits)) {
-                if (__any_sync(0xffffffffu, mx >= 0x7ff0000000000000ULL)) {
-                    ctl |= SKT_BAD;
+                if (__any_sync(0xffffffffu, mx >= SK_NONFINITE_BITS)) {
+                    ctl |= SK_BAD;
                 } else {
                     // absorption: u = v = 1/K in POT == divide the scaled iterates by K; remember 1/ut, 1/vt
                     bool r = false;
@@ -200,12 +180,12 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
                         if (row_ok[rr]) {
                             rea[rr] = 1.0 / u[rr];
                             reb[rr] = 1.0 / v[rr];
-                            r |= !(u[rr] > 1e-250 && u[rr] < 1e250 && v[rr] > 1e-250 && v[rr] < 1e250);
+                            r |= sk_out_of_range(u[rr], v[rr]);
                             u[rr] *= invK;
                             v[rr] *= invK;
                         }
                     ++nabs;
-                    if (__any_sync(0xffffffffu, r)) ctl |= SKT_BAD;
+                    if (__any_sync(0xffffffffu, r)) ctl |= SK_BAD;
                 }
             }
         }
@@ -228,35 +208,25 @@ sinkhorn_tail_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
                 c = fma(vb[j], w0 + w1, c);
             }
             const double cost = warp_sum_d(c);
-            if (lane == 0) {
-                out[w] = cost;
-                if (iters_out) iters_out[w] = ii;
-                if (abs_out) abs_out[w] = nabs;
-                if (status_out) status_out[w] = status;
-            }
+            if (lane == 0) sk_store(res, w, status, cost, ii, nabs);
         } else if (lane == 0) {
-            const unsigned long long slot = atomicAdd(n_redo, 1ULL);
-            if ((long long)slot < SK_REDO_CAP) redo_list[slot] = w;
-            out[w] = __longlong_as_double(SK_REDO_MARK);
-            if (status_out) status_out[w] = -1;
+            sk_store(res, w, status, 0.0, ii, nabs);
         }
         __syncwarp();
     }
 }
 
 template <int KP, bool SYM>
-static int skt_launch_t(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
-                        const double *scratch, const SkTail &tail, unsigned long long *tail_counter, double *out,
-                        int *iters, int *absn, int *status, long long *redo, unsigned long long *n_redo,
+static int skt_launch_t(const double *props, int K, const SkParams &prm, const PairMap &pm, const SkSetup &s,
+                        const double *scratch, const SkTail &tail, unsigned long long *tail_counter, const SkOut &res,
                         cudaStream_t st)
 {
     const size_t smem = sizeof(double) * ((size_t)(SYM ? 2 : 3) * KP * KP + (size_t)SKT_WARPS * 3 * KP);
     PILOT_CUDA(cudaFuncSetAttribute(sinkhorn_tail_kernel<KP, SYM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)smem));
-    const double *K0 = setup, *K0T = K0 + KP * KP, *MK = K0T + KP * KP, *c0 = MK + KP * KP;
-    const int *asym = reinterpret_cast<const int *>(setup + 3 * KP * KP + KP);
     sinkhorn_tail_kernel<KP, SYM><<<sm_count(), SKT_WARPS * 32, smem, st>>>(
-        props, K, prm, pm, K0, K0T, MK, c0, asym, scratch, tail, tail_counter, out, iters, absn, status, redo, n_redo);
+        props, K, prm, pm, s, scratch, tail, tail_counter, res.out, res.iters, res.absn, res.status, res.redo,
+        res.n_redo);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
@@ -264,18 +234,13 @@ static int skt_launch_t(const double *props, int K, const SkParams &prm, const P
 // continues the problems the panel kernel handed over (none: the CTAs return at once)
 int skt_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
                const double *scratch, bool symmetric, const SkTail &tail, unsigned long long *tail_counter,
-               double *out, int *iters, int *absn, int *status, long long *redo, unsigned long long *n_redo,
-               cudaStream_t st)
+               const SkOut &res, cudaStream_t st)
 {
     const int KP = skb_pad(K);
-#define SKT_GO(KPV)                                                                                              \
-    do {                                                                                                         \
-        if (symmetric)                                                                                           \
-            return skt_launch_t<KPV, true>(props, K, prm, pm, setup, scratch, tail, tail_counter, out, iters,     \
-                                           absn, status, redo, n_redo, st);                                      \
-        return skt_launch_t<KPV, false>(props, K, prm, pm, setup, scratch, tail, tail_counter, out, iters, absn,  \
-                                        status, redo, n_redo, st);                                               \
-    } while (0)
+    const SkSetup s = sk_setup_view(setup, KP);
+#define SKT_GO(KPV) \
+    return (symmetric ? skt_launch_t<KPV, true> : skt_launch_t<KPV, false>)(props, K, prm, pm, s, scratch, tail, \
+                                                                            tail_counter, res, st)
     if (KP == 16) SKT_GO(16);
     if (KP == 32) SKT_GO(32);
     if (KP == 48) SKT_GO(48);

@@ -15,18 +15,6 @@ namespace pilot {
 
 constexpr int SWK_WARPS = 8;
 
-// branch-free x / y for finite positive y: 20-bit seed r, e = 1 - y r, q = x r (1 + e + e^2): relative
-// error e^3 ~ 2^-60 before the final rounding, a dependent chain of MUFU + 3 FP64 ops (the chain
-// length, not the op count, is what a lone warp pays for)
-__device__ __forceinline__ double swk_div(double x, double y)
-{
-    double r;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(y));
-    const double e = fma(-y, r, 1.0);
-    const double q0 = x * r;
-    return fma(q0, fma(e, e, e), q0);
-}
-
 // sum_i k0[i] * buf[i]; buf is read as 128-bit broadcasts; 8 independent chains of KP / 8 FMAs and a
 // 3-level tree (16 chains would save one more dependent op but spill at KP = 32)
 template <int KP>
@@ -44,21 +32,19 @@ __device__ __forceinline__ double swk_matvec(const double (&k0)[KP], const doubl
     return ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
 }
 
-enum { SWK_PEND = 1, SWK_FORCE = 2, SWK_BAD = 4 };
-
 template <int KP>
 __global__ void __launch_bounds__(SWK_WARPS * 32, 2)
-sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, PairMap pm,
-                     const double *__restrict__ gK0, const double *__restrict__ gMK,
-                     const int *__restrict__ asym_flag, double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
-                     int *__restrict__ status_out, unsigned long long *__restrict__ counter,
-                     long long *__restrict__ redo_list, unsigned long long *__restrict__ n_redo)
+sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, PairMap pm, SkSetup s,
+                     unsigned long long *__restrict__ counter, double *__restrict__ out, int *__restrict__ iters_out,
+                     int *__restrict__ abs_out, int *__restrict__ status_out, long long *__restrict__ redo_list,
+                     unsigned long long *__restrict__ n_redo)
 {
+    const SkOut res{out, iters_out, abs_out, status_out, redo_list, n_redo};
     __shared__ double sMK[KP * KP];                             // M o K0, for the final cost
     __shared__ __align__(16) double sbuf[SWK_WARPS][2][KP];    // per warp: broadcast copies of ut, vt
-    if (*asym_flag != 0) return;  // asymmetric cost: the panel kernel enqueued behind this one runs instead
+    if (*s.asym != 0) return;  // asymmetric cost: the panel kernel enqueued behind this one runs instead
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int e = threadIdx.x; e < KP * KP; e += blockDim.x) sMK[e] = gMK[e];
+    for (int e = threadIdx.x; e < KP * KP; e += blockDim.x) sMK[e] = s.MK[e];
     __syncthreads();
 
     const int j = lane;
@@ -66,9 +52,9 @@ sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
     const int jc = in_pad ? j : 0;
     double k0[KP];  // column j of K0 (== row j: the cost is symmetric)
 #pragma unroll
-    for (int i = 0; i < KP; ++i) k0[i] = in_pad ? gK0[i * KP + jc] : 0.0;
+    for (int i = 0; i < KP; ++i) k0[i] = in_pad ? s.K0[i * KP + jc] : 0.0;
     double *ub = sbuf[warp][0], *vb = sbuf[warp][1];
-    const unsigned long long tau_bits = (unsigned long long)__double_as_longlong(prm.tau);
+    const long long tau_bits = __double_as_longlong(prm.tau);
     const double invK = 1.0 / K;
 
     for (;;) {
@@ -83,7 +69,7 @@ sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
         // ut, vt >= 0 always; rea = 1 / ut, reb = 1 / vt at the last absorption (1 before the first)
         double u = row_ok ? invK : 0.0, v = u, rea = 1.0, reb = 1.0;
         int ii = 0, nabs = 0, status = PILOT_ST_MAXITER;
-        int ctl = 0;               // what the next round has to resolve: SWK_PEND | SWK_FORCE | SWK_BAD
+        int ctl = 0;               // what the next round has to resolve: SK_PEND | SK_FORCE | SK_BAD
         int until_check = 0;       // iterations until the next convergence check (ii % check_every == 0)
         for (;;) {
             // ---- T = K0^T ut, then resolve the check / cap of the previous iteration ----
@@ -91,50 +77,44 @@ sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
             __syncwarp();
             const double T = swk_matvec<KP>(k0, ub);
             if (ctl) {
-                if (ctl & SWK_BAD) { status = -1; break; }
+                if (ctl & SK_BAD) { status = -1; break; }
                 bool conv = false;
-                if (ctl & SWK_PEND) {
+                if (ctl & SK_PEND) {
                     const double d = row_ok ? fma(v, T, -b) : 0.0;
                     conv = sqrt(warp_sum_d(d * d)) <= prm.stop_thr;
                 }
                 if (conv) { status = PILOT_ST_CONVERGED; break; }
-                if (ctl & SWK_FORCE) { status = PILOT_ST_MAXITER; break; }
+                if (ctl & SK_FORCE) { status = PILOT_ST_MAXITER; break; }
             }
             // ---- vt = b / T ----
-            v = row_ok ? swk_div(b, T) : 0.0;
+            v = row_ok ? sk_div(b, T) : 0.0;
             if (in_pad) vb[j] = v;
             __syncwarp();
             // ---- ut = a / (K0 vt) ----
             const double S = swk_matvec<KP>(k0, vb);
-            u = row_ok ? swk_div(a, S) : 0.0;
-            // u, v of the reference = ut * rea, vt * reb: absorb when one exceeds tau; NaN / Inf (and
-            // anything negative) compare above every finite positive value as unsigned bit patterns
-            const unsigned long long bu = (unsigned long long)__double_as_longlong(u * rea);
-            const unsigned long long bv = (unsigned long long)__double_as_longlong(v * reb);
-            const unsigned long long mx = bu > bv ? bu : bv;
-            ctl = (until_check == 0) ? SWK_PEND : 0;
-            until_check = (until_check == 0 ? prm.check_every : until_check) - 1;
-            ++ii;
-            if (ii >= prm.num_iter_max) ctl |= SWK_FORCE;
+            u = row_ok ? sk_div(a, S) : 0.0;
+            // u, v of the reference = ut * rea, vt * reb: absorb when one exceeds tau
+            const long long mx = max(sk_abs_bits(u * rea), sk_abs_bits(v * reb));
+            ctl = sk_step(prm, until_check, ii);
             if (__any_sync(0xffffffffu, mx > tau_bits)) {
-                if (__any_sync(0xffffffffu, mx >= 0x7ff0000000000000ULL)) {
-                    ctl |= SWK_BAD;  // NaN or Inf somewhere in u, v
+                if (__any_sync(0xffffffffu, mx >= SK_NONFINITE_BITS)) {
+                    ctl |= SK_BAD;  // NaN or Inf somewhere in u, v
                 } else {
                     // absorption: u = v = 1/K in POT == divide the scaled iterates by K; remember 1/ut, 1/vt
                     bool r = false;
                     if (row_ok) {
                         rea = 1.0 / u;
                         reb = 1.0 / v;
-                        // keep e^{+-alpha/reg} comfortably inside the FP64 range
-                        r = !(u > 1e-250 && u < 1e250 && v > 1e-250 && v < 1e250);
+                        r = sk_out_of_range(u, v);
                         u *= invK;
                         v *= invK;
                     }
                     ++nabs;
-                    if (__any_sync(0xffffffffu, r)) ctl |= SWK_BAD;
+                    if (__any_sync(0xffffffffu, r)) ctl |= SK_BAD;
                 }
             }
         }
+        double cost = 0.0;
         if (status >= 0) {
             // cost = sum_j vt_j * sum_i (M o K0)_ij ut_i   (ub holds the current ut)
             double c0 = 0.0, c1 = 0.0;
@@ -145,19 +125,9 @@ sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
                     c1 = fma(sMK[(i + 1) * KP + j], ub[i + 1], c1);
                 }
             }
-            const double cost = warp_sum_d(v * (c0 + c1));
-            if (lane == 0) {
-                out[w] = cost;
-                if (iters_out) iters_out[w] = ii;
-                if (abs_out) abs_out[w] = nabs;
-                if (status_out) status_out[w] = status;
-            }
-        } else if (lane == 0) {
-            const unsigned long long slot = atomicAdd(n_redo, 1ULL);
-            if ((long long)slot < SK_REDO_CAP) redo_list[slot] = (long long)w;
-            out[w] = __longlong_as_double(SK_REDO_MARK);
-            if (status_out) status_out[w] = -1;
+            cost = warp_sum_d(v * (c0 + c1));
         }
+        if (lane == 0) sk_store(res, (long long)w, status, cost, ii, nabs);
         __syncwarp();
     }
 }
@@ -165,21 +135,19 @@ sinkhorn_warp_kernel(const double *__restrict__ props, int K, SkParams prm, Pair
 int swk_max_k() { return 32; }
 
 // `setup` must already hold the output of skb_setup (symmetric cost only)
-int swk_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup, double *out,
-               int *iters, int *absn, int *status, unsigned long long *counter, long long *redo,
-               unsigned long long *n_redo, cudaStream_t st)
+int swk_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
+               const SkOut &res, unsigned long long *counter, cudaStream_t st)
 {
     const int KP = skb_pad(K);
-    const double *K0 = setup, *MK = setup + 2 * KP * KP;
-    const int *asym = reinterpret_cast<const int *>(setup + 3 * KP * KP + KP);
+    const SkSetup s = sk_setup_view(setup, KP);
     long long ctas = pm.n_local;  // spread a small batch over all SMs, one problem per warp at a time
     if (ctas > 2LL * sm_count()) ctas = 2LL * sm_count();
     if (KP == 16)
-        sinkhorn_warp_kernel<16><<<(int)ctas, SWK_WARPS * 32, 0, st>>>(props, K, prm, pm, K0, MK, asym, out, iters, absn,
-                                                                       status, counter, redo, n_redo);
+        sinkhorn_warp_kernel<16><<<(int)ctas, SWK_WARPS * 32, 0, st>>>(props, K, prm, pm, s, counter, res.out, res.iters,
+                                                                       res.absn, res.status, res.redo, res.n_redo);
     else
-        sinkhorn_warp_kernel<32><<<(int)ctas, SWK_WARPS * 32, 0, st>>>(props, K, prm, pm, K0, MK, asym, out, iters, absn,
-                                                                       status, counter, redo, n_redo);
+        sinkhorn_warp_kernel<32><<<(int)ctas, SWK_WARPS * 32, 0, st>>>(props, K, prm, pm, s, counter, res.out, res.iters,
+                                                                       res.absn, res.status, res.redo, res.n_redo);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
