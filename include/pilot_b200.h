@@ -146,16 +146,20 @@ int pilot_cdist(const double *centroids_f64, int K, int D, int metric,
  * algo: 0 = shared-Gibbs-kernel solvers (fast path: one warp per problem with K0
  *           in registers for K <= 32 and a symmetric cost, else 8-problem DMMA
  *           panels whose stragglers are finished by a warp-form tail kernel;
- *           problems the scaled form cannot represent are re-solved by the
- *           reference-form kernel, however many they are),
- *       1 = reference-form kernel only (per-problem Gibbs kernel, literal schedule),
- *       3 = DMMA-panel solver (+ tail) for every K <= 64.
- * K > 64 (up to ~150) always takes the reference-form kernel.  The call is fully
+ *           65 <= K <= 256: DMMA panels with K0 split in row stripes over a
+ *           thread-block cluster; problems the scaled form cannot represent are
+ *           re-solved by the reference-form kernel, however many they are),
+ *       1 = reference-form kernel only (per-problem Gibbs kernel, literal schedule;
+ *           the Gibbs matrix lives in the workspace when it does not fit shared
+ *           memory, K > ~155),
+ *       3 = DMMA-panel solver (+ tail) for every K <= 64, the cluster panels above.
+ * 1 <= K <= 256 (ot.sinkhorn2 itself has no limit).  The call is fully
  * asynchronous on `stream` (whether the cost is symmetric is decided on the
  * device: both variants of a solver are enqueued, one returns at once).
  * precision: PILOT_F64 = the schedule above in double (within 1e-9 of POT);
  * PILOT_F32 = log-domain Sinkhorn in float (within 1e-4; stop_thr is raised to
- * what float can resolve), any K <= 64.
+ * what float can resolve) for K <= 64; K > 64 runs the FP64 solvers whatever
+ * the precision.
  */
 int pilot_sinkhorn_pairs(const double *props, int S, int K, const double *cost,
                          double reg, int num_iter_max, double stop_thr,

@@ -1,7 +1,8 @@
-// C-ABI entry of kernel (3): dispatch between the batched shared-Gibbs-kernel solver and
+// C-ABI entry of kernel (3): dispatch between the batched shared-Gibbs-kernel solvers and
 // the reference-form kernel (reference call site: pilotpy/tools/Trajectory.py:513-515).
 #include <stdint.h>
 #include <stdlib.h>
+#include <algorithm>
 #include "sinkhorn.cuh"
 
 namespace pilot {
@@ -22,10 +23,12 @@ struct SkWorkspace {
     long long *redo;
     SkTailRec *tail_rec;
     double *tail_uv;
-    size_t bytes;  // end of the last region
+    double *gibbs;  // the reference-form kernel's Gibbs matrices when they do not fit shared memory
+    size_t bytes;   // end of the last region
 };
 
-// carves the workspace at `base` (nullptr: only its size)
+// carves the workspace at `base` (nullptr: only its size).  Up to 64 types every region is what the panel kernels
+// need; above, the setup buffer has the extent roundup(K, 8), and the scratch also holds the wide kernel's rea / reb.
 static SkWorkspace sk_workspace(void *base, int K)
 {
     const int KP = skb_pad(K <= 64 ? K : 64);
@@ -34,11 +37,14 @@ static SkWorkspace sk_workspace(void *base, int K)
     const auto take = [&p](size_t bytes) { const uintptr_t r = p; p += bytes; return r; };
     SkWorkspace ws;
     ws.ctr = (SkCounters *)take(256);
-    ws.setup = (double *)take(skb_setup_bytes(KP));
-    ws.scratch = (double *)take(skb_scratch_bytes(KP, sm_count()));
+    ws.setup = (double *)take(skb_setup_bytes(sk_setup_extent(K)));
+    const size_t wide_scratch = K > 64 ? skw_scratch_bytes(sm_count()) : 0;
+    ws.scratch = (double *)take(std::max(skb_scratch_bytes(KP, sm_count()), wide_scratch));
     ws.redo = (long long *)take((size_t)SK_REDO_CAP * sizeof(long long));
     ws.tail_rec = (SkTailRec *)take((tail_slots * sizeof(SkTailRec) + 255) / 256 * 256);
     ws.tail_uv = (double *)take(tail_slots * 2 * KP * sizeof(double));
+    const size_t gibbs = sinkhorn_ref_gibbs_bytes(K);
+    ws.gibbs = gibbs ? (double *)take(gibbs) : nullptr;
     ws.bytes = p - (uintptr_t)base;
     return ws;
 }
@@ -56,12 +62,12 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
 {
     using namespace pilot;
     PILOT_CHECK_ARG(props && cost && out && workspace, "pilot_sinkhorn_pairs: NULL pointer");
-    PILOT_CHECK_ARG(S >= 1 && K >= 1, "pilot_sinkhorn_pairs: S=%d K=%d", S, K);
+    PILOT_CHECK_ARG(S >= 1, "pilot_sinkhorn_pairs: S=%d", S);
+    PILOT_CHECK_ARG(K >= 1 && K <= 256, "pilot_sinkhorn_pairs: K=%d outside the supported range [1, 256]", K);
     PILOT_CHECK_ARG(reg > 0.0, "pilot_sinkhorn_pairs: reg must be > 0");
     PILOT_CHECK_ARG(num_iter_max >= 1 && check_every >= 1, "pilot_sinkhorn_pairs: bad iteration parameters");
     PILOT_CHECK_ARG(algo == 0 || algo == 1 || algo == 3, "pilot_sinkhorn_pairs: algo %d", algo);
     PILOT_CHECK_ARG(precision == PILOT_F64 || precision == PILOT_F32, "pilot_sinkhorn_pairs: precision=%d", precision);
-    PILOT_CHECK_ARG(sinkhorn_ref_smem(K) <= 200 * 1024, "pilot_sinkhorn_pairs: K=%d too large (max ~150)", K);
     const SkWorkspace ws = sk_workspace(workspace, K);
     PILOT_CHECK_ARG(workspace_bytes >= ws.bytes, "pilot_sinkhorn_pairs: workspace %zu < %zu bytes", workspace_bytes,
                     ws.bytes);
@@ -74,19 +80,32 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     const SkOut res{out, iters, absorptions, status, ws.redo, &ws.ctr->n_redo};
 
     PILOT_CUDA(cudaMemsetAsync(ws.ctr, 0, sizeof(SkCounters), st));
-    if (algo == 1 || K > 64) return sinkhorn_ref_launch(props, K, cost, prm, pm, res, SK_SOLVE_ALL, &ws.ctr->slow, st);
+    if (algo == 1)
+        return sinkhorn_ref_launch(props, K, cost, prm, pm, res, SK_SOLVE_ALL, &ws.ctr->slow, ws.gibbs, st);
     long long redo_cap = SK_REDO_CAP;
     // (PILOT_SK_REDO_CAP, tests only: a smaller list capacity, to exercise the overflow scan)
     if (const char *e = getenv("PILOT_SK_REDO_CAP")) {
         const long long v = atoll(e);
         if (v >= 0 && v < redo_cap) redo_cap = v;
     }
+    if (K > 64) {
+        // 65..256 types, FP64 whatever the precision: DMMA panels with K0 split over a cluster (both variants are
+        // enqueued, the setup kernel's asymmetry flag picks one on the device), then the reference form for
+        // the problems the scaled form cannot carry
+        rc = skb_setup(cost, K, prm, ws.setup, st);
+        if (rc) return rc;
+        for (int sym = 1; sym >= 0; --sym) {
+            rc = skw_launch(props, K, prm, pm, ws.setup, ws.scratch, sym != 0, res, &ws.ctr->fast, st);
+            if (rc) return rc;
+        }
+        return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, ws.gibbs, st);
+    }
     if (precision == PILOT_F32) {
         // single precision: per-problem kernel in registers (sinkhorn_f32.cu); what it cannot carry (NaN/Inf,
         // zero masses) goes to the FP64 reference-form kernel like in the FP64 mode
         rc = skf_launch(props, K, cost, prm, pm, res, &ws.ctr->fast, st);
         if (rc) return rc;
-        return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, st);
+        return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, ws.gibbs, st);
     }
     // evict_max measured: 0 (no hand-over) 2.23 ms, 2: 1.45 ms, 4: 1.44 ms, 7: 1.56 ms for 10^4 problems at K = 64
     const SkTail tail{ws.tail_rec, ws.tail_uv, &ws.ctr->n_tail, 2};
@@ -127,5 +146,5 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
         if (rc) return rc;
     }
     // problems the scaled form could not represent (normally none): reference-form kernel
-    return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, st);
+    return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, ws.gibbs, st);
 }

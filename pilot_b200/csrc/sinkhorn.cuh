@@ -1,5 +1,5 @@
 // Shared declarations and device helpers of the Sinkhorn kernels (sinkhorn_ref.cu, sinkhorn_batched.cu,
-// sinkhorn_tail.cu, sinkhorn_warp.cu, sinkhorn_f32.cu).
+// sinkhorn_tail.cu, sinkhorn_warp.cu, sinkhorn_f32.cu, sinkhorn_wide.cu).
 #pragma once
 #include "common.cuh"
 
@@ -27,8 +27,8 @@ struct SkOut {
     unsigned long long *n_redo;
 };
 
-// the setup buffer skb_setup fills (sk_setup_view): K0, K0^T, M o K0 (KP x KP each, zero padded), c0 = K0^T (1/K),
-// and a flag that is != 0 when M differs from its transpose; the solver kernels read the flag themselves
+// the setup buffer skb_setup fills (sk_setup_view): K0, K0^T, M o K0 (KP x KP each, zero padded, KP =
+// sk_setup_extent(K)), c0 = K0^T (1/K), and a flag that is != 0 when M differs from its transpose; the solver kernels read the flag themselves
 struct SkSetup {
     const double *K0, *K0T, *MK, *c0;
     const int *asym;
@@ -102,13 +102,18 @@ __device__ __forceinline__ void sk_store(const SkOut &res, long long w, int stat
 }
 
 size_t sinkhorn_ref_smem(int K);
+// workspace the reference-form kernel needs for its Gibbs matrices: 0 while they fit shared memory
+size_t sinkhorn_ref_gibbs_bytes(int K);
 // redo_cap: SK_SOLVE_ALL, or solve the problems queued in res.redo (at most redo_cap of them are listed; the rest is
-// found by their marker)
+// found by their marker).  gibbs: sinkhorn_ref_gibbs_bytes(K) bytes of workspace (nullptr when that is 0).
 constexpr long long SK_SOLVE_ALL = -1;
 int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
-                        const SkOut &res, long long redo_cap, unsigned long long *counter, cudaStream_t st);
+                        const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
+                        cudaStream_t st);
 
 int skb_pad(int K);
+// storage extent of the setup buffer: skb_pad(K) up to 64 types, roundup(K, 8) above
+int sk_setup_extent(int K);
 size_t skb_setup_bytes(int KP);
 SkSetup sk_setup_view(const double *setup, int KP);
 size_t skb_smem_bytes(int KP);
@@ -130,6 +135,12 @@ int skt_launch(const double *props, int K, const SkParams &prm, const PairMap &p
 int swk_max_k();
 int swk_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
                const SkOut &res, unsigned long long *counter, cudaStream_t st);
+
+// 65 <= K <= 256: DMMA panels with K0 split in row stripes over a thread-block cluster (sinkhorn_wide.cu);
+// scratch: skw_scratch_bytes(sm_count()) bytes
+size_t skw_scratch_bytes(int ctas);
+int skw_launch(const double *props, int K, const SkParams &prm, const PairMap &pm, const double *setup,
+               double *scratch, bool symmetric, const SkOut &res, unsigned long long *counter, cudaStream_t st);
 
 // FP32 mode: one warp per problem, per-problem kernel in registers (sinkhorn_f32.cu), K <= 64
 int skf_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,

@@ -439,6 +439,7 @@ size_t skb_scratch_bytes(int KP, int ctas)
 }
 // padded problem size: the DMMA tiles need a multiple of 8, the work grows with KP^2
 int skb_pad(int K) { return K <= 16 ? 16 : (K <= 32 ? 32 : (K <= 48 ? 48 : 64)); }
+int sk_setup_extent(int K) { return K <= 64 ? skb_pad(K) : (K + 7) / 8 * 8; }
 int skb_slots_per_cta() { return SKB_WARPS * SKB_SPW; }
 int skb_slots_per_warp() { return SKB_SPW; }
 int skb_warps() { return SKB_WARPS; }
@@ -461,7 +462,7 @@ static int skb_launch_t(const double *props, int K, const SkParams &prm, const P
 // fills the buffer sk_setup_view describes
 int skb_setup(const double *cost, int K, const SkParams &prm, double *setup, cudaStream_t st)
 {
-    const int KP = skb_pad(K);
+    const int KP = sk_setup_extent(K);
     const SkSetup s = sk_setup_view(setup, KP);
     int *asym = const_cast<int *>(s.asym);
     PILOT_CUDA(cudaMemsetAsync(asym, 0, sizeof(int), st));

@@ -8,13 +8,17 @@
 //   err <= stop_thr; NaN -> roll back to the previous (u, v); cap num_iter_max;
 //   result sum(M * Gamma).
 // One CTA of roundup(K, 32) >= 64 threads per problem (thread t owns row t and column t),
-// persistent CTAs pulling problems from a global counter.  This is the always-valid path: the batched
-// shared-kernel solver (sinkhorn_batched.cu) hands it the problems it cannot represent.
+// persistent CTAs pulling problems from a global counter.  Up to K ~ 155 the Gibbs matrix sits in shared memory;
+// above, each CTA keeps it in its own slice of the workspace (GK), at most one CTA per SM so that the slices
+// stay few (K = 256: 514 KB each, 78 MB on 148 SMs, which should mostly stay in the 126 MB L2; not measured).
+// This is the always-valid path: the batched shared-kernel solvers (sinkhorn_batched.cu, sinkhorn_wide.cu) hand
+// it the problems they cannot represent.
 #include "sinkhorn.cuh"
 
 namespace pilot {
 
-constexpr int SKR_MAX_WARPS = 8;   // K <= 256 by construction; the shared-memory check admits K <= ~150
+constexpr int SKR_MAX_WARPS = 8;   // K <= 256 by construction
+constexpr size_t SKR_SMEM_MAX = 200 * 1024;  // larger Gibbs matrices go to the workspace
 constexpr int SKR_SCAN = 256;      // problems per work item of the marker scan (mode 2)
 
 static int skr_threads(int K) { return K <= 64 ? 64 : ((K + 31) / 32) * 32; }
@@ -44,17 +48,19 @@ __device__ __forceinline__ double block_sum64(double v, double *red)
 // mode 0: every local problem; mode 1: the problems of the redo list (at most max_list of them); mode 2: only if
 // more than max_list problems were queued (the list overflowed): scan out[] for the redo marker the fast
 // kernels left behind and solve those (the listed ones were overwritten by mode 1 already).
+// GK: the Gibbs matrix lives in the CTA's slice of `gibbs` (K x (K | 1) doubles) instead of shared memory.
+template <bool GK>
 __global__ void __launch_bounds__(SKR_MAX_WARPS * 32)
 sinkhorn_ref_kernel(const double *__restrict__ props, int K, const double *__restrict__ M, SkParams prm,
                     PairMap pm, int mode, const long long *__restrict__ list,
                     const unsigned long long *__restrict__ n_list_dev, long long max_list,
                     double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
-                    int *__restrict__ status_out, unsigned long long *__restrict__ counter)
+                    int *__restrict__ status_out, unsigned long long *__restrict__ counter, double *gibbs)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int KS = K | 1;  // odd row stride: row- and column-walks are both conflict-free
-    double *Km = reinterpret_cast<double *>(smem_raw);
-    double *u = Km + (size_t)K * KS, *v = u + K, *up = v + K, *vp = up + K;
+    double *Km = GK ? gibbs + (size_t)blockIdx.x * K * KS : reinterpret_cast<double *>(smem_raw);
+    double *u = GK ? reinterpret_cast<double *>(smem_raw) : Km + (size_t)K * KS, *v = u + K, *up = v + K, *vp = up + K;
     double *al = vp + K, *be = al + K, *lu = be + K, *lv = lu + K, *red = lv + K;
     __shared__ long long s_l;
     __shared__ int s_nfound;
@@ -200,29 +206,37 @@ size_t sinkhorn_ref_smem(int K)
     const int KS = K | 1;
     return sizeof(double) * ((size_t)K * KS + 8 * (size_t)K + SKR_MAX_WARPS);
 }
+static bool skr_global_gibbs(int K) { return sinkhorn_ref_smem(K) > SKR_SMEM_MAX; }
+size_t sinkhorn_ref_gibbs_bytes(int K)
+{
+    return skr_global_gibbs(K) ? sizeof(double) * (size_t)sm_count() * K * (K | 1) : 0;
+}
 
 int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
-                        const SkOut &res, long long redo_cap, unsigned long long *counter, cudaStream_t st)
+                        const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
+                        cudaStream_t st)
 {
     const bool queued = redo_cap != SK_SOLVE_ALL;
     // with a device-side list the amount of work is unknown here: launch one wave and let the CTAs loop
     const long long n_work = queued ? (long long)sm_count() * 4 : pm.n_local;
     if (n_work <= 0) return 0;
-    const size_t smem = sinkhorn_ref_smem(K);
+    const bool gk = skr_global_gibbs(K);
+    PILOT_CHECK_ARG(!gk || gibbs, "sinkhorn reference-form kernel: K=%d needs a Gibbs workspace", K);
+    const size_t smem = gk ? sizeof(double) * (8 * (size_t)K + SKR_MAX_WARPS) : sinkhorn_ref_smem(K);
     const int threads = skr_threads(K);
     PILOT_CHECK_ARG(threads <= SKR_MAX_WARPS * 32, "sinkhorn reference-form kernel: K=%d too large", K);
-    PILOT_CUDA(cudaFuncSetAttribute(sinkhorn_ref_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const auto kern = gk ? sinkhorn_ref_kernel<true> : sinkhorn_ref_kernel<false>;
+    PILOT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
-    PILOT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sinkhorn_ref_kernel, threads, smem));
-    if (per_sm < 1) per_sm = 1;
+    PILOT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+    if (per_sm < 1 || gk) per_sm = 1;  // gibbs holds one slice per SM
     long long ctas = (long long)sm_count() * per_sm;
     if (ctas > n_work) ctas = n_work;
     // modes 1 and 2 run back to back on the stream and share the counter: reset it before each
     for (int mode = queued ? 1 : 0; mode <= (queued ? 2 : 0); ++mode) {
         PILOT_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-        sinkhorn_ref_kernel<<<(unsigned)ctas, threads, smem, st>>>(props, K, cost, prm, pm, mode, res.redo, res.n_redo,
-                                                                  redo_cap, res.out, res.iters, res.absn, res.status,
-                                                                  counter);
+        kern<<<(unsigned)ctas, threads, smem, st>>>(props, K, cost, prm, pm, mode, res.redo, res.n_redo, redo_cap,
+                                                    res.out, res.iters, res.absn, res.status, counter, gibbs);
         PILOT_LAUNCH_CHECK();
     }
     return 0;
