@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PILOT_B200_ABI_VERSION 2
+#define PILOT_B200_ABI_VERSION 3
 
 /* element types of the embedding handed to pilot_centroid_median; also the `precision`
  * of the two pair solvers (FP64 = the 1e-9 parity tier, FP32 = the 1e-4 tier) */
@@ -47,9 +47,15 @@ extern "C" {
 #define PILOT_METRIC_SEUCLIDEAN  9   /* V = var(centroids, axis=0, ddof=1), SciPy's default */
 #define PILOT_METRIC_HAMMING     10
 
-/* how a linear problem index g maps to a sample pair (i, j) */
+/* how a linear problem index g maps to a sample pair (i, j); S = rows of props */
 #define PILOT_PAIRS_FULL  0   /* g = i*S + j, all S*S ordered pairs incl. diagonal     */
 #define PILOT_PAIRS_UPPER 1   /* strictly upper triangle, row-major, S*(S-1)/2 pairs    */
+/* two sample sets concatenated in props: rows i = 0..S_a-1 against columns
+ * j = S_a + j', j' = 0..S_b-1 (S_b = S - S_a); g = i*S_b + j', S_a*S_b pairs, the
+ * problem (a = props[i], b = props[S_a + j']).  S_a travels in pilot_pair_range.rows.
+ * A problem is solved by the same arithmetic as the same pair of the FULL / UPPER
+ * square over props, so a block is bit-identical to those entries of the square. */
+#define PILOT_PAIRS_RECT  2
 
 /* per-problem status written by the *_pairs kernels */
 #define PILOT_ST_CONVERGED 0  /* Sinkhorn: err <= stopThr ; EMD: optimal               */
@@ -71,12 +77,13 @@ extern "C" {
  * (SURVEY.md 8e)
  */
 typedef struct {
-    int64_t total;   /* problems in the window: first + total <= S*S (FULL) or S*(S-1)/2 (UPPER) */
+    int64_t total;   /* problems in the window: first + total <= S*S (FULL), S*(S-1)/2 (UPPER)
+                        or S_a*(S - S_a) (RECT) */
     int64_t block;   /* problems per block (>=1) */
     int32_t nranks;
     int32_t rank;
     int32_t mode;    /* PILOT_PAIRS_* */
-    int32_t reserved;
+    int32_t rows;    /* row count S_a in PILOT_PAIRS_RECT (1 <= S_a < S), 0 otherwise */
     int64_t first;   /* linear index of the window's first problem */
 } pilot_pair_range;
 
@@ -153,6 +160,11 @@ int pilot_cdist(const double *centroids_f64, int K, int D, int metric,
  *           the Gibbs matrix lives in the workspace when it does not fit shared
  *           memory, K > ~155),
  *       3 = DMMA-panel solver (+ tail) for every K <= 64, the cluster panels above.
+ * Solver selection for algo = 0: the warp form runs for a symmetric cost when
+ * 17 <= K <= 32, or K <= 16 and S*S < 200000, with S the rows of props (in
+ * PILOT_PAIRS_RECT the concatenated sets, so a block is solved as the square over
+ * them solves it); every other choice depends on K only.  It never depends on the
+ * window, the rank or the partition, so results are bit-identical under them.
  * 1 <= K <= 256 (ot.sinkhorn2 itself has no limit).  The call is fully
  * asynchronous on `stream` (whether the cost is symmetric is decided on the
  * device: both variants of a solver are enqueued, one returns at once).
@@ -186,10 +198,13 @@ int pilot_emd_pairs(const double *props, int S, int K, const double *cost,
 
 /*
  * (5) Packed per-rank results (as laid out by an all-gather: rank r's chunk at
- * packed + r*chunk_stride) -> dense S x S row-major matrix, EMD[i,j] with
- * i = row sample (a), j = column sample (b) as Trajectory.py:511/515.
- * UPPER mode mirrors into the lower triangle and writes `diag_value` on the
- * diagonal.
+ * packed + r*chunk_stride) -> dense row-major matrix, EMD[i,j] with
+ * i = row sample (a), j = column sample (b) as Trajectory.py:511/515.  Shape of
+ * `dense` per mode (a window writes only its own entries):
+ *   FULL : S x S;
+ *   UPPER: S x S, mirrored into the lower triangle, `diag_value` on the diagonal;
+ *   RECT : S_a x (S - S_a), dense[i*(S - S_a) + j'] = problem (i, S_a + j'); no
+ *          mirror, no diagonal.
  */
 int pilot_unpack_pairs(const double *packed, int64_t chunk_stride, int S,
                        const pilot_pair_range *range, double diag_value,

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # PILOT_B200_LIB: another build of the same library (A/B measurements of kernel variants only)
 LIB_PATH = os.environ.get("PILOT_B200_LIB") or os.path.join(_HERE, "csrc", "libpilot_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # constants mirrored from include/pilot_b200.h
 F32, F64 = 0, 1
@@ -23,7 +23,7 @@ METRICS = {"cosine": 0, "cos": 0, "euclidean": 1, "euclid": 1, "eu": 1, "e": 1, 
            "correlation": 5, "co": 5,
            "braycurtis": 6, "canberra": 7, "minkowski": 8, "mi": 8, "m": 8, "pnorm": 8,
            "seuclidean": 9, "se": 9, "s": 9, "hamming": 10, "hamm": 10, "ha": 10, "h": 10, "matching": 10}
-PAIRS_FULL, PAIRS_UPPER = 0, 1
+PAIRS_FULL, PAIRS_UPPER, PAIRS_RECT = 0, 1, 2
 PRECISIONS = {"f64": F64, "fp64": F64, "float64": F64, "double": F64,
               "f32": F32, "fp32": F32, "float32": F32, "single": F32}
 
@@ -49,10 +49,12 @@ EXPORTS = (
 
 
 class PairRange(ctypes.Structure):
-    """pilot_pair_range (include/pilot_b200.h)."""
+    """pilot_pair_range (include/pilot_b200.h).  ``rows``: the row count S_a in PAIRS_RECT, 0 otherwise;
+    ``reserved`` is its former name and still accepted."""
     _fields_ = [("total", ctypes.c_int64), ("block", ctypes.c_int64), ("nranks", ctypes.c_int32),
-                ("rank", ctypes.c_int32), ("mode", ctypes.c_int32), ("reserved", ctypes.c_int32),
+                ("rank", ctypes.c_int32), ("mode", ctypes.c_int32), ("rows", ctypes.c_int32),
                 ("first", ctypes.c_int64)]
+    reserved = property(lambda self: self.rows, lambda self, v: setattr(self, "rows", v))
 
 
 class PilotLibraryError(RuntimeError):

@@ -37,9 +37,13 @@ int make_pair_map(const pilot_pair_range *r, int S, PairMap *pm)
     PILOT_CHECK_ARG(r->block >= 1, "pair range: block must be >= 1 (got %lld)", (long long)r->block);
     PILOT_CHECK_ARG(r->nranks >= 1 && r->rank >= 0 && r->rank < r->nranks,
                     "pair range: bad rank %d of %d", r->rank, r->nranks);
-    PILOT_CHECK_ARG(r->mode == PILOT_PAIRS_FULL || r->mode == PILOT_PAIRS_UPPER,
+    PILOT_CHECK_ARG(r->mode == PILOT_PAIRS_FULL || r->mode == PILOT_PAIRS_UPPER || r->mode == PILOT_PAIRS_RECT,
                     "pair range: bad mode %d", r->mode);
-    long long cap = r->mode == PILOT_PAIRS_FULL ? (long long)S * S : (long long)S * (S - 1) / 2;
+    const bool rect = r->mode == PILOT_PAIRS_RECT;
+    PILOT_CHECK_ARG(!rect || (r->rows >= 1 && r->rows < S),
+                    "pair range: RECT row count %d outside [1, %d)", r->rows, S);
+    long long cap = rect ? (long long)r->rows * (S - r->rows)
+                         : r->mode == PILOT_PAIRS_FULL ? (long long)S * S : (long long)S * (S - 1) / 2;
     PILOT_CHECK_ARG(r->first >= 0 && r->total >= 0 && r->first + r->total <= cap,
                     "pair range: window [%lld, +%lld) outside [0, %lld]", (long long)r->first, (long long)r->total, cap);
     pm->total = r->total;
@@ -49,6 +53,8 @@ int make_pair_map(const pilot_pair_range *r, int S, PairMap *pm)
     pm->rank = r->rank;
     pm->mode = r->mode;
     pm->S = S;
+    pm->row_len = rect ? S - r->rows : S;
+    pm->col0 = rect ? r->rows : 0;
     pm->n_local = range_count(r->total, r->block, r->nranks, r->rank);
     return 0;
 }

@@ -42,6 +42,9 @@ struct PairMap {
     long long total, block, first;
     int nranks, rank, mode, S;
     long long n_local;
+    // FULL and RECT rows: g = i*row_len + (j - col0).  FULL: (S, 0), RECT: (S - S_a, S_a); UPPER: (S, 0), the
+    // dense matrix's row length
+    int row_len, col0;
 };
 
 __host__ __device__ inline long long range_count(long long total, long long block, int nranks, int rank)
@@ -83,9 +86,9 @@ __device__ __forceinline__ void upper_to_ij(long long g, int S, int &i, int &j)
 __device__ __forceinline__ void global_to_ij(const PairMap &pm, long long g, int &i, int &j)
 {
     g += pm.first;
-    if (pm.mode == PILOT_PAIRS_FULL) {
-        i = (int)(g / pm.S);
-        j = (int)(g - (long long)i * pm.S);
+    if (pm.mode != PILOT_PAIRS_UPPER) {  // FULL, RECT
+        i = (int)(g / pm.row_len);
+        j = pm.col0 + (int)(g - (long long)i * pm.row_len);
     } else {
         upper_to_ij(g, pm.S, i, j);
     }

@@ -124,6 +124,7 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     // large batch goes to the DMMA panels instead (measured: 400 K problems, K = 12: 5.6 vs 6.9 ms).
     // The choice depends on the COHORT size only (not on this rank's share or on the window), so that a problem is
     // solved by the same arithmetic however the pair space is partitioned: results are partition-invariant bit for bit.
+    // In RECT mode S is the concatenation of the two sets, so a block takes the choice of the square over them.
     const bool warp_form = algo == 0 && K <= swk_max_k() && (K > 16 || (long long)S * S < 200000);
     if (warp_form) {  // symmetric cost only; an asymmetric one falls through to the general panels below
         rc = swk_launch(props, K, prm, pm, ws.setup, res, &ws.ctr->fast, st);

@@ -1,5 +1,6 @@
 // Kernel (5): packed per-rank results -> dense S x S matrix (EMD[i, j], i = row sample),
-// mirroring the upper triangle for the symmetric exact-EMD case.  Replaces the NumPy
+// mirroring the upper triangle for the symmetric exact-EMD case, or the dense S_a x S_b block of
+// the RECT pair space (never mirrored: its rows and columns are different samples).  Replaces the NumPy
 // element assignments EMD[i, j] = ... of the reference loop (pilotpy/tools/Trajectory.py:511,515).
 // HBM-bound: 8 B read + 8 (or 16) B written per problem.
 #include "common.cuh"
@@ -18,7 +19,7 @@ __global__ void unpack_kernel(const double *__restrict__ packed, long long chunk
         const double v = packed[(long long)owner * chunk_stride + local];
         int i, j;
         global_to_ij(pm, g, i, j);
-        dense[(long long)i * S + j] = v;
+        dense[(long long)i * pm.row_len + (j - pm.col0)] = v;
         if (pm.mode == PILOT_PAIRS_UPPER) dense[(long long)j * S + i] = v;
     }
     if (pm.mode == PILOT_PAIRS_UPPER)

@@ -47,14 +47,19 @@ def _workspace(nbytes: int, device) -> torch.Tensor:
     return buf
 
 
-def make_range(total: int, mode: int, nranks: int = 1, rank: int = 0, block: Optional[int] = None) -> PairRange:
+def make_range(total: int, mode: int, nranks: int = 1, rank: int = 0, block: Optional[int] = None,
+               rows: int = 0, first: int = 0) -> PairRange:
+    """rows: the row count S_a of the PAIRS_RECT space (0 for FULL / UPPER)."""
     if block is None:
         block = max(1, min(4096, -(-total // (nranks * 4)))) if nranks > 1 else max(1, total)
     return PairRange(total=int(total), block=int(block), nranks=int(nranks), rank=int(rank), mode=int(mode),
-                     reserved=0)
+                     rows=int(rows), first=int(first))
 
 
-def n_pairs(S: int, mode: int) -> int:
+def n_pairs(S: int, mode: int, rows: int = 0) -> int:
+    """Problems in the pair space of S samples (PAIRS_RECT: S_a = rows against the other S - rows)."""
+    if mode == _lib.PAIRS_RECT:
+        return rows * (S - rows)
     return S * S if mode == _lib.PAIRS_FULL else S * (S - 1) // 2
 
 
@@ -196,11 +201,12 @@ def emd_pairs(props: torch.Tensor, cost: torch.Tensor, rng: PairRange, max_pivot
 
 def unpack_pairs(packed: torch.Tensor, chunk_stride: int, S: int, rng: PairRange, diag_value: float = 0.0,
                  dense: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """All-gathered packed chunks -> dense S x S float64 matrix."""
+    """All-gathered packed chunks -> dense float64 matrix: S x S, or S_a x (S - S_a) for PAIRS_RECT."""
     _require_cuda(packed)
     assert packed.dtype == torch.float64 and packed.is_contiguous()
     if dense is None:
-        dense = torch.empty((S, S), dtype=torch.float64, device=packed.device)
+        shape = (rng.rows, S - rng.rows) if rng.mode == _lib.PAIRS_RECT else (S, S)
+        dense = torch.empty(shape, dtype=torch.float64, device=packed.device)
     check(lib().pilot_unpack_pairs(_ptr(packed), int(chunk_stride), S, ctypes.byref(rng), float(diag_value),
                                    _ptr(dense), _stream()), "pilot_unpack_pairs")
     return dense

@@ -12,6 +12,10 @@ exact-EMD case) into the dense S x S matrix on every rank.
                       matrix rows; band b's rows cross PCIe on a copy stream while band b+1
                       is being solved, so the 3.2 GB of a 20 000-sample matrix cost no time
                       on top of the kernels.
+``cross_pairs`` / ``cross_pairs_host`` -> the S_a x S_b block between two sample sets (the RECT
+                      pair space over their concatenation), on the device / in host memory.
+``extend_pairs``   -> the entries a matrix over S_old samples lacks once S_new samples join.
+Every block is bit-identical to the same entries of the square over the concatenated samples.
 
 Replaces the double loop of the reference's ``wasserstein_d``
 (/root/reference/pilotpy/tools/Trajectory.py:505-515).
@@ -59,9 +63,12 @@ def global_to_local(g: int, block: int, nranks: int) -> Tuple[int, int]:
     return b % nranks, (b // nranks) * block + off
 
 
-def global_to_ij(g: int, S: int, mode: int) -> Tuple[int, int]:
+def global_to_ij(g: int, S: int, mode: int, rows: int = 0) -> Tuple[int, int]:
     if mode == _lib.PAIRS_FULL:
         return divmod(g, S)
+    if mode == _lib.PAIRS_RECT:  # rows 0..rows-1 against columns rows..S-1
+        i, jp = divmod(g, S - rows)
+        return i, rows + jp
     i = 0
     # rows before i hold i*(2S-i-1)/2 entries
     lo, hi = 0, S - 2
@@ -75,30 +82,40 @@ def global_to_ij(g: int, S: int, mode: int) -> Tuple[int, int]:
     return i, g - i * (2 * S - i - 1) // 2 + i + 1
 
 
-def row_start(i: int, S: int, mode: int) -> int:
-    """Linear index of the first problem of matrix row i (i == S: one past the end)."""
+def row_start(i: int, S: int, mode: int, rows: int = 0) -> int:
+    """Linear index of the first problem of matrix row i (i == number of rows: one past the end)."""
+    if mode == _lib.PAIRS_RECT:
+        return i * (S - rows)
     return i * S if mode == _lib.PAIRS_FULL else i * (2 * S - i - 1) // 2
 
 
-def band_rows(S: int, mode: int, n_bands: int) -> List[int]:
-    """Row boundaries r_0 = 0 < r_1 < ... < r_B = S of bands holding about the same number of problems
-    (upper-triangle rows get shorter, so later bands take more rows)."""
-    total = row_start(S, S, mode) if mode == _lib.PAIRS_FULL else S * (S - 1) // 2
-    n_bands = max(1, min(n_bands, S))
+def band_rows(S: int, mode: int, n_bands: int, rows: int = 0) -> List[int]:
+    """Row boundaries r_0 = 0 < r_1 < ... < r_B = R of bands holding about the same number of problems
+    (upper-triangle rows get shorter, so later bands take more rows).  R = S, or `rows` in PAIRS_RECT."""
+    total = ops.n_pairs(S, mode, rows)
+    R = rows if mode == _lib.PAIRS_RECT else S
+    n_bands = max(1, min(n_bands, R))
     edges = [0]
     for b in range(1, n_bands):
         target = total * b // n_bands
-        lo, hi = edges[-1], S
+        lo, hi = edges[-1], R
         while lo < hi:  # first row whose start is >= target
             mid = (lo + hi) // 2
-            if row_start(mid, S, mode) >= target:
+            if row_start(mid, S, mode, rows) >= target:
                 hi = mid
             else:
                 lo = mid + 1
-        if lo > edges[-1] and lo < S:
+        if lo > edges[-1] and lo < R:
             edges.append(lo)
-    edges.append(S)
+    edges.append(R)
     return edges
+
+
+def sinkhorn_form_changes(S_a: int, S_b: int, K: int) -> bool:
+    """True when pilot_sinkhorn_pairs picks different solvers for cohorts of S_a and of S_b samples: for K <= 16
+    the warp form runs when S*S < 200 000 and the DMMA panels otherwise (sinkhorn.cu).  The two agree within a few
+    ulp but not bit for bit, so a matrix solved at one size is not a block of the square at the other."""
+    return K <= 16 and (S_a * S_a < 200_000) != (S_b * S_b < 200_000)
 
 
 def choose_block(total: int, nranks: int) -> int:
@@ -129,8 +146,10 @@ def cost_is_symmetric_metric_like(cost) -> bool:
     return bool(((c == c.t()).all() & (torch.diagonal(c) == 0).all() & (c >= 0).all()).item())
 
 
-def _mode_for(regularized, cost_norm, symmetric: Optional[bool]) -> Tuple[bool, int]:
+def _mode_for(regularized, cost_norm, symmetric: Optional[bool], rect: bool = False) -> Tuple[bool, int]:
     exact = isinstance(regularized, str) and regularized == "unreg"
+    if rect:  # a block between two sample sets holds no mirrored pair, whatever the cost
+        return exact, _lib.PAIRS_RECT
     if exact:
         if symmetric is None:
             symmetric = cost_is_symmetric_metric_like(cost_norm)
@@ -140,12 +159,12 @@ def _mode_for(regularized, cost_norm, symmetric: Optional[bool]) -> Tuple[bool, 
 
 def _solve_window(props, cost_norm, exact: bool, reg: float, mode: int, first: int, total: int, nranks: int,
                   rank: int, group, algo: int, precision, dense: torch.Tensor, want_info: bool = False,
-                  marks: Optional[list] = None):
+                  marks: Optional[list] = None, rows: int = 0):
     """Solve the window [first, first + total) of the pair space over the ranks, all-gather, unpack into
-    `dense`.  Everything is asynchronous on the current stream."""
+    `dense` (rows: S_a of PAIRS_RECT).  Everything is asynchronous on the current stream."""
     S = props.shape[0]
     block = choose_block(total, nranks)
-    rng = PairRange(total=total, block=block, nranks=nranks, rank=rank, mode=mode, reserved=0, first=first)
+    rng = PairRange(total=total, block=block, nranks=nranks, rank=rank, mode=mode, rows=rows, first=first)
     chunk = max(1, range_count(total, block, nranks, 0))  # rank 0 always holds the largest share
     packed = torch.zeros((chunk,), dtype=torch.float64, device=props.device) if nranks > 1 else None
 
@@ -179,24 +198,26 @@ def _solve_window(props, cost_norm, exact: bool, reg: float, mode: int, first: i
 
 def all_pairs(props: torch.Tensor, cost_norm: torch.Tensor, regularized="unreg", reg: float = 0.1,
               group=None, algo: int = 0, symmetric: Optional[bool] = None, want_info: bool = False,
-              precision="f64", single_rank: bool = False, marks: Optional[list] = None):
+              precision="f64", single_rank: bool = False, marks: Optional[list] = None, rows: int = 0):
     """Dense S x S matrix EMD[i, j] = OT(props[i], props[j]) on every rank (device tensor).
 
     regularized == "unreg" -> exact EMD, anything else -> stabilised Sinkhorn
     (the string comparison is the reference's, Trajectory.py:507).
     single_rank=True solves everything on this rank, whatever the process group (parity checks).
     marks: optional list receiving (name, cuda event) pairs around solve / gather / unpack.
+    rows > 0: only the rows x (S - rows) block of props[:rows] against props[rows:] (PAIRS_RECT).
     """
     S, K = props.shape
     nranks, rank = (1, 0) if single_rank else world(group)
-    exact, mode = _mode_for(regularized, cost_norm, symmetric)
-    total = ops.n_pairs(S, mode)
+    exact, mode = _mode_for(regularized, cost_norm, symmetric, rect=rows > 0)
+    shape = (rows, S - rows) if rows > 0 else (S, S)
+    total = ops.n_pairs(S, mode, rows)
     if total == 0:
-        dense = torch.zeros((S, S), dtype=torch.float64, device=props.device)
+        dense = torch.zeros(shape, dtype=torch.float64, device=props.device)
         return (dense, None) if want_info else dense
-    dense = torch.empty((S, S), dtype=torch.float64, device=props.device)
+    dense = torch.empty(shape, dtype=torch.float64, device=props.device)
     info = _solve_window(props, cost_norm, exact, reg, mode, 0, total, nranks, rank, group, algo, precision, dense,
-                         want_info, marks)
+                         want_info, marks, rows)
     if want_info:
         return dense, info
     return dense
@@ -214,7 +235,7 @@ def _copy_stream(dev: torch.device) -> "torch.cuda.Stream":
 
 def all_pairs_host(props: torch.Tensor, cost_norm: torch.Tensor, regularized="unreg", reg: float = 0.1,
                    group=None, algo: int = 0, symmetric: Optional[bool] = None, precision="f64",
-                   n_bands: Optional[int] = None, with_transpose: bool = False
+                   n_bands: Optional[int] = None, with_transpose: bool = False, rows: int = 0
                    ) -> Tuple[np.ndarray, Optional[np.ndarray]]:
     """The dense S x S matrix in HOST memory on every rank, and optionally an independent ndarray holding
     its transpose (the reference hands out the ndarray and a DataFrame of the transpose, Trajectory.py:518).
@@ -225,12 +246,17 @@ def all_pairs_host(props: torch.Tensor, cost_norm: torch.Tensor, regularized="un
     later bands run.  With the upper-triangle mode a band's rows are final once it is unpacked (their
     left part was mirrored in by the earlier bands) and the transpose is the matrix itself; otherwise the
     transpose is formed on the device after the last band and copied out then.
+    rows > 0: only the rows x (S - rows) block of props[:rows] against props[rows:] (PAIRS_RECT); the bands
+    are rows of the block, and with_transpose does not apply.
     """
     S, K = props.shape
     nranks, rank = world(group)
-    exact, mode = _mode_for(regularized, cost_norm, symmetric)
-    total = ops.n_pairs(S, mode)
-    out = np.empty((S, S), dtype=np.float64)
+    if rows > 0 and with_transpose:
+        raise ValueError("all_pairs_host: with_transpose is not available for a block (rows > 0)")
+    exact, mode = _mode_for(regularized, cost_norm, symmetric, rect=rows > 0)
+    shape = (rows, S - rows) if rows > 0 else (S, S)
+    total = ops.n_pairs(S, mode, rows)
+    out = np.empty(shape, dtype=np.float64)
     out_T = np.empty((S, S), dtype=np.float64) if with_transpose else None
     if S == 0 or total == 0:
         out[...] = 0.0
@@ -240,17 +266,18 @@ def all_pairs_host(props: torch.Tensor, cost_norm: torch.Tensor, regularized="un
     dev = props.device
     if n_bands is None:
         # small matrices: one band (the copy takes microseconds); big ones: ~256 MB of rows per band
-        n_bands = max(1, min(64, (S * S * 8) >> 28))
-    edges = band_rows(S, mode, n_bands)
-    dense = torch.empty((S, S), dtype=torch.float64, device=dev)
+        n_bands = max(1, min(64, (shape[0] * shape[1] * 8) >> 28))
+    edges = band_rows(S, mode, n_bands, rows)
+    dense = torch.empty(shape, dtype=torch.float64, device=dev)
     main = torch.cuda.current_stream(dev)
     side = _copy_stream(dev)
     done = []
     for b in range(len(edges) - 1):
-        first = row_start(edges[b], S, mode)
-        cnt = row_start(edges[b + 1], S, mode) - first
+        first = row_start(edges[b], S, mode, rows)
+        cnt = row_start(edges[b + 1], S, mode, rows) - first
         if cnt > 0:
-            _solve_window(props, cost_norm, exact, reg, mode, first, cnt, nranks, rank, group, algo, precision, dense)
+            _solve_window(props, cost_norm, exact, reg, mode, first, cnt, nranks, rank, group, algo, precision, dense,
+                          rows=rows)
         else:  # the last row of the upper triangle holds no pair: only its diagonal entry
             dense[edges[b]:edges[b + 1]].diagonal(offset=edges[b]).zero_()
         ev = torch.cuda.Event()
@@ -277,3 +304,67 @@ def all_pairs_host(props: torch.Tensor, cost_norm: torch.Tensor, regularized="un
             dense_T.record_stream(side)
     dense.record_stream(side)
     return out, out_T
+
+
+def _concat(props_a: torch.Tensor, props_b: torch.Tensor) -> torch.Tensor:
+    if props_a.shape[1] != props_b.shape[1]:
+        raise ValueError(f"the two sample sets have {props_a.shape[1]} and {props_b.shape[1]} cell types")
+    return torch.cat([props_a, props_b]).contiguous()
+
+
+def cross_pairs(props_a: torch.Tensor, props_b: torch.Tensor, cost_norm: torch.Tensor, regularized="unreg",
+                reg: float = 0.1, group=None, algo: int = 0, want_info: bool = False, precision="f64",
+                single_rank: bool = False):
+    """Dense S_a x S_b matrix D[i, j] = OT(props_a[i], props_b[j]) on every rank (device tensor): the RECT pair
+    space over the concatenated sets, partitioned and all-gathered as in all_pairs.  Bit-identical to the same
+    entries of all_pairs over torch.cat([props_a, props_b])."""
+    S_a, S_b = props_a.shape[0], props_b.shape[0]
+    if S_a == 0 or S_b == 0:
+        dense = torch.zeros((S_a, S_b), dtype=torch.float64, device=props_a.device)
+        return (dense, None) if want_info else dense
+    return all_pairs(_concat(props_a, props_b), cost_norm, regularized, reg, group, algo, want_info=want_info,
+                     precision=precision, single_rank=single_rank, rows=S_a)
+
+
+def cross_pairs_host(props_a: torch.Tensor, props_b: torch.Tensor, cost_norm: torch.Tensor, regularized="unreg",
+                     reg: float = 0.1, group=None, algo: int = 0, precision="f64",
+                     n_bands: Optional[int] = None) -> np.ndarray:
+    """cross_pairs with the result in HOST memory, through the band pipeline of all_pairs_host."""
+    S_a, S_b = props_a.shape[0], props_b.shape[0]
+    if S_a == 0 or S_b == 0:
+        return np.zeros((S_a, S_b), dtype=np.float64)
+    out, _ = all_pairs_host(_concat(props_a, props_b), cost_norm, regularized, reg, group, algo, precision=precision,
+                            n_bands=n_bands, rows=S_a)
+    return out
+
+
+def extend_pairs(props_old: torch.Tensor, props_new: torch.Tensor, cost_norm: torch.Tensor, regularized="unreg",
+                 reg: float = 0.1, group=None, algo: int = 0, symmetric: Optional[bool] = None, precision="f64",
+                 single_rank: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+    """What the square over S = S_old + S_new samples holds beyond its S_old x S_old corner, solving only
+    those problems: (old_new [S_old, S_new], new_rows [S_new, S]) on every rank (device tensors), the rows
+    S_old.. and the columns S_old.. of rows 0..S_old-1 of all_pairs(torch.cat([props_old, props_new])),
+    bit for bit.
+
+    old x new is the RECT block.  The rows of the new samples are the window of the square's own pair space
+    that holds them, over the concatenated samples, so every problem runs as the square runs it.  Where the
+    square mirrors its upper triangle (exact EMD, symmetric cost) that window holds new x new only, and
+    new x old is the transposed old x new block."""
+    S_old, S_new = props_old.shape[0], props_new.shape[0]
+    props = _concat(props_old, props_new)
+    S = S_old + S_new
+    nranks, rank = (1, 0) if single_rank else world(group)
+    exact, mode = _mode_for(regularized, cost_norm, symmetric)
+    old_new = cross_pairs(props_old, props_new, cost_norm, regularized, reg, group, algo, precision=precision,
+                          single_rank=single_rank)
+    # unpack addresses the window's entries in the S x S matrix; only rows S_old.. are read back
+    dense = torch.empty((S, S), dtype=torch.float64, device=props.device)
+    first = row_start(S_old, S, mode)
+    total = ops.n_pairs(S, mode) - first
+    if total > 0:
+        _solve_window(props, cost_norm, exact, reg, mode, first, total, nranks, rank, group, algo, precision, dense)
+    new_rows = dense[S_old:]
+    if mode == _lib.PAIRS_UPPER:
+        new_rows[:, :S_old] = old_new.t()
+        new_rows[:, S_old:].diagonal().zero_()  # unpack writes it too, but not when one new sample leaves no pair
+    return old_new, new_rows

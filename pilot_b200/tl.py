@@ -523,14 +523,20 @@ def _check_emd_inputs(P: np.ndarray, cost: np.ndarray) -> None:
                              "a and b vector must have the same sum")
 
 
+def _stack_props(Clu_rep) -> Tuple[list, np.ndarray]:
+    """(sample ids, proportions [S, K] float64) of a {sample: proportions} dict."""
+    ids = list(Clu_rep.keys())
+    if not ids:
+        return ids, np.zeros((0, 0))
+    return ids, np.ascontiguousarray(np.stack([np.asarray(Clu_rep[s], dtype=np.float64) for s in ids]))
+
+
 def wasserstein_d(Clu_rep, cost, regularized="unreg", reg=0.1, precision="f64"):
     """All ordered sample pairs: exact EMD (``regularized == "unreg"``) or stabilised
     Sinkhorn (anything else).  Returns ``(EMD ndarray [S,S], DataFrame indexed by sampleID)``.
     ``precision`` is an extension of the reference signature: "f64" (default, within 1e-9 of POT) or
     "f32" (single-precision solvers, within 1e-4)."""
-    samples_id = list(Clu_rep.keys())
-    P = np.ascontiguousarray(np.stack([np.asarray(Clu_rep[s], dtype=np.float64) for s in samples_id])) \
-        if samples_id else np.zeros((0, 0))
+    samples_id, P = _stack_props(Clu_rep)
     C = np.ascontiguousarray(np.asarray(cost, dtype=np.float64))
     if len(samples_id) == 0:
         EMD = np.zeros((0, 0))
@@ -542,6 +548,83 @@ def wasserstein_d(Clu_rep, cost, regularized="unreg", reg=0.1, precision="f64"):
     EMD, EMD_T = pairs.all_pairs_host(_to_device(P), _to_device(C), regularized, reg, symmetric=sym,
                                       with_transpose=True, precision=precision)
     return EMD, _emd_frame(EMD, samples_id, EMD_T)
+
+
+
+
+def _check_two_sets(P_a: np.ndarray, P_b: np.ndarray, C: np.ndarray, regularized) -> None:
+    """Checks of wasserstein_d_cross / _extend made before any device work: the same number of cell types in
+    both sets and the cost, and under "unreg" equal masses across both sets (_check_emd_inputs)."""
+    if P_a.shape[1] != P_b.shape[1]:
+        raise ValueError(f"the two sample sets have {P_a.shape[1]} and {P_b.shape[1]} cell types")
+    if C.shape != (P_a.shape[1], P_a.shape[1]):
+        raise ValueError(f"cost has shape {C.shape}, expected {P_a.shape[1]} x {P_a.shape[1]} (one row and "
+                         "column per cell type)")
+    if regularized == "unreg":
+        _check_emd_inputs(np.concatenate([P_a, P_b]), C)
+
+
+def wasserstein_d_cross(Clu_rep_a, Clu_rep_b, cost, regularized="unreg", reg=0.1, precision="f64"):
+    """OT costs between two sample sets that share the cell types and the cost matrix, for example a
+    discovery and a validation cohort: exact EMD (``regularized == "unreg"``) or stabilised Sinkhorn.
+
+    Returns ``(D ndarray [S_a, S_b], DataFrame)`` with ``D[i, j]`` the cost of (a_i, b_j); the frame is
+    indexed by the ids of ``Clu_rep_a`` (index name ``sampleID``) and its columns are the ids of
+    ``Clu_rep_b`` (not transposed).  Only the S_a x S_b problems are solved, and ``D`` is bit-identical to
+    the same entries of ``wasserstein_d({**Clu_rep_a, **Clu_rep_b}, cost, ...)`` when the ids are distinct."""
+    ids_a, P_a = _stack_props(Clu_rep_a)
+    ids_b, P_b = _stack_props(Clu_rep_b)
+    if ids_a and ids_b:
+        C = np.ascontiguousarray(np.asarray(cost, dtype=np.float64))
+        _check_two_sets(P_a, P_b, C, regularized)
+        D = pairs.cross_pairs_host(_to_device(P_a), _to_device(P_b), _to_device(C), regularized, reg,
+                                   precision=precision)
+    else:
+        D = np.zeros((len(ids_a), len(ids_b)))
+    frame = pd.DataFrame(D.copy(), index=pd.Index(ids_a, name="sampleID"), columns=pd.Index(ids_b))
+    return D, frame
+
+
+def wasserstein_d_extend(Clu_rep, EMD, Clu_rep_new, cost, regularized="unreg", reg=0.1, precision="f64"):
+    """Extend the matrix ``EMD`` of the samples ``Clu_rep`` with the samples ``Clu_rep_new``.
+
+    Returns ``(EMD, EMD_df)`` over old ∪ new (old samples first), bit-identical to
+    ``wasserstein_d({**Clu_rep, **Clu_rep_new}, cost, regularized, reg, precision)``, frame included, while
+    solving only the problems that involve a new sample: old x new and new x new, and new x old unless the
+    exact solver mirrors (symmetric cost), as the square does.  Sinkhorn with K <= 16 solves the whole union
+    instead when the old cohort is below 448 samples and the union is not (the solver changes there).  ``EMD`` must be this library's
+    ``wasserstein_d(Clu_rep, cost, ...)`` output with the same arguments; that is not checked (only its shape
+    is), and the old corner is copied as given.  An id present in both sets raises."""
+    ids_old, P_old = _stack_props(Clu_rep)
+    ids_new, P_new = _stack_props(Clu_rep_new)
+    if not ids_old:
+        return wasserstein_d(Clu_rep_new, cost, regularized, reg, precision)
+    if not ids_new:
+        EMD = np.array(EMD, dtype=np.float64)
+        return EMD, _emd_frame(EMD, ids_old)
+    shared = set(ids_old).intersection(ids_new)
+    if shared:
+        raise ValueError(f"wasserstein_d_extend: sample ids in both sets: {sorted(map(str, shared))[:5]}")
+    EMD = np.asarray(EMD, dtype=np.float64)
+    S_old, S_new = len(ids_old), len(ids_new)
+    if EMD.shape != (S_old, S_old):
+        raise ValueError(f"EMD is {EMD.shape}, expected ({S_old}, {S_old}) for the samples of Clu_rep")
+    C = np.ascontiguousarray(np.asarray(cost, dtype=np.float64))
+    _check_two_sets(P_old, P_new, C, regularized)
+    if regularized != "unreg" and pairs.sinkhorn_form_changes(S_old, S_old + S_new, C.shape[0]):
+        # the union crosses the cohort size at which Sinkhorn changes solver for K <= 16, so EMD's bits are not
+        # those of the union's square: solve it all (S_old <= 447 here, at most 200 000 extra problems)
+        return wasserstein_d({**Clu_rep, **Clu_rep_new}, cost, regularized, reg, precision)
+    sym = pairs.cost_is_symmetric_metric_like(C) if regularized == "unreg" else None
+    old_new, new_rows = pairs.extend_pairs(_to_device(P_old), _to_device(P_new), _to_device(C), regularized, reg,
+                                           symmetric=sym, precision=precision)
+    S = S_old + S_new
+    out = np.empty((S, S), dtype=np.float64)
+    out[:S_old, S_old:] = old_new.cpu().numpy()
+    out[S_old:] = new_rows.cpu().numpy()
+    out[:S_old, :S_old] = EMD
+    # the square's frame takes its transpose; a mirrored matrix is its own transpose
+    return out, _emd_frame(out, ids_old + ids_new, out.copy() if sym else None)
 
 
 # ---------------------------------------------------------------------------
