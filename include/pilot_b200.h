@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PILOT_B200_ABI_VERSION 3
+#define PILOT_B200_ABI_VERSION 4
 
 /* element types of the embedding handed to pilot_centroid_median; also the `precision`
  * of the two pair solvers (FP64 = the 1e-9 parity tier, FP32 = the 1e-4 tier) */
@@ -195,6 +195,39 @@ int pilot_emd_pairs(const double *props, int S, int K, const double *cost,
                     int precision, double *out, int32_t *status,
                     int32_t *pivots, void *workspace, size_t workspace_bytes,
                     void *stream);
+
+/*
+ * (3p, 4p) Transport plans of the n problems a caller lists -- what ot.sinkhorn
+ * (method="sinkhorn_stabilized") and ot.emd return beside the costs of (3) and (4).
+ * Problem l is (a = props[pair_a[l]], b = props[pair_b[l]]), solved as given (no
+ * mirroring), on one device, in FP64:
+ *   plans[l*K*K + r*K + c] = Gamma[r, c]  (n x K x K; row r: a cell type of a,
+ *                                          column c: a cell type of b)
+ *   out[l]                 = the cost, computed by the code that writes it in the
+ *                            pair solvers above
+ * pilot_emd_plans runs the exact solver of pilot_emd_pairs (bit-mask up to 64 types,
+ * general network simplex above); Gamma holds the basis flows (at most 2K - 1
+ * non-zeros), its rows sum to a and its columns to emd2's rescaled b.
+ * pilot_sinkhorn_plans runs the reference-form kernel of pilot_sinkhorn_pairs
+ * (algo = 1), whose cost it reproduces bit for bit; Gamma is
+ * exp(-(M - alpha_i - beta_j)/reg + log u_i + log v_j), POT's statement.
+ * 1 <= K <= 256, n >= 0.  status, iters and absorptions may be NULL.  A pair index
+ * outside [0, S) is never read: that problem gets a NaN cost, a NaN plan and
+ * PILOT_ST_NUMERIC.  Workspace: pilot_workspace_bytes(PILOT_WS_EMD, n, K, S, 0),
+ * resp. PILOT_WS_SINKHORN.  Asynchronous on `stream`.
+ */
+int pilot_emd_plans(const double *props, int S, int K, const double *cost,
+                    int64_t max_pivots, const int32_t *pair_a,
+                    const int32_t *pair_b, int64_t n, double *plans,
+                    double *out, int32_t *status, void *workspace,
+                    size_t workspace_bytes, void *stream);
+int pilot_sinkhorn_plans(const double *props, int S, int K, const double *cost,
+                         double reg, int num_iter_max, double stop_thr,
+                         double tau, int check_every, const int32_t *pair_a,
+                         const int32_t *pair_b, int64_t n, double *plans,
+                         double *out, int32_t *iters, int32_t *absorptions,
+                         int32_t *status, void *workspace,
+                         size_t workspace_bytes, void *stream);
 
 /*
  * (5) Packed per-rank results (as laid out by an all-gather: rank r's chunk at

@@ -16,8 +16,8 @@ from . import _lib, h5ad, ops, pairs, pl, tl  # noqa: F401
 from .tl import (Cluster_Representations, Precomputed_distance, Sil_computing, cost_matrix,  # noqa: F401
                  extract_data_anno_pathomics_from_h5ad, extract_data_anno_scRNA_from_h5ad, load_h5ad,
                  return_real_labels,
-                 set_path_for_results, wasserstein_d, wasserstein_d_cross, wasserstein_d_extend,
-                 wasserstein_distance)
+                 set_path_for_results, transport_plan, wasserstein_d, wasserstein_d_cross, wasserstein_d_extend,
+                 wasserstein_distance, wasserstein_plans)
 
 __version__ = "0.1.0"
 

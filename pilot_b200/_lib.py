@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # PILOT_B200_LIB: another build of the same library (A/B measurements of kernel variants only)
 LIB_PATH = os.environ.get("PILOT_B200_LIB") or os.path.join(_HERE, "csrc", "libpilot_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # constants mirrored from include/pilot_b200.h
 F32, F64 = 0, 1
@@ -43,8 +43,8 @@ SIL_PRECOMPUTED = 100
 EXPORTS = (
     "pilot_abi_version", "pilot_last_error", "pilot_range_count", "pilot_workspace_bytes", "pilot_launch_count",
     "pilot_hist", "pilot_props_finalize", "pilot_centroid_median", "pilot_cdist",
-    "pilot_sinkhorn_pairs", "pilot_emd_pairs", "pilot_unpack_pairs", "pilot_knn_rows", "pilot_silhouette_rows",
-    "pilot_pipe_peak",
+    "pilot_sinkhorn_pairs", "pilot_emd_pairs", "pilot_sinkhorn_plans", "pilot_emd_plans", "pilot_unpack_pairs",
+    "pilot_knn_rows", "pilot_silhouette_rows", "pilot_pipe_peak",
 )
 
 
@@ -99,6 +99,11 @@ def lib():
                                        vp, sz, vp]
     L.pilot_emd_pairs.restype = i32
     L.pilot_emd_pairs.argtypes = [vp, i32, i32, vp, i64, prp, i32, vp, vp, vp, vp, sz, vp]
+    L.pilot_sinkhorn_plans.restype = i32
+    L.pilot_sinkhorn_plans.argtypes = [vp, i32, i32, vp, dbl, i32, dbl, dbl, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp,
+                                       sz, vp]
+    L.pilot_emd_plans.restype = i32
+    L.pilot_emd_plans.argtypes = [vp, i32, i32, vp, i64, vp, vp, i64, vp, vp, vp, vp, sz, vp]
     L.pilot_unpack_pairs.restype = i32
     L.pilot_unpack_pairs.argtypes = [vp, i64, i32, prp, dbl, vp, vp]
     L.pilot_knn_rows.restype = i32

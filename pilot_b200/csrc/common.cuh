@@ -96,6 +96,39 @@ __device__ __forceinline__ void global_to_ij(const PairMap &pm, long long g, int
 
 int make_pair_map(const pilot_pair_range *r, int S, PairMap *pm);
 
+// ---- transport plans (pilot_emd_plans, pilot_sinkhorn_plans) ------------------
+// The extra arguments of a solver's plan variant: problem l is (a = props[pair_a[l]], b = props[pair_b[l]]) and its
+// K x K plan goes to plans + l*K*K, row-major (rows: a's types).  The instances without a plan take the empty
+// specialisation, so that their parameters and their code stay exactly as they were.
+template <bool PLAN> struct PlanArgs {};
+template <> struct PlanArgs<true> {
+    const int *pair_a, *pair_b;
+    int S;
+    double *plans;
+};
+
+// (si, sj) of problem l; false when an index lies outside [0, S): that problem reads nothing and gets a NaN plan,
+// a NaN cost and PILOT_ST_NUMERIC
+__device__ __forceinline__ bool plan_pair(const PlanArgs<true> &pa, long long l, int &si, int &sj)
+{
+    si = pa.pair_a[l];
+    sj = pa.pair_b[l];
+    return si >= 0 && si < pa.S && sj >= 0 && sj < pa.S;
+}
+constexpr long long PILOT_NAN_BITS = 0x7ff8000000000000LL;
+
+// the pair map of a plan call: n problems, l = 0..n-1 (no pair space behind it)
+inline PairMap plan_pair_map(long long n, int S)
+{
+    PairMap pm{};
+    pm.total = n;
+    pm.block = n > 0 ? n : 1;
+    pm.nranks = 1;
+    pm.S = S;
+    pm.n_local = n;
+    return pm;
+}
+
 // ---- warp helpers -----------------------------------------------------------
 __device__ __forceinline__ double shfl_d(double v, int src)
 {

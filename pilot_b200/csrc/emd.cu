@@ -239,13 +239,15 @@ __device__ __noinline__ int emd_pivot_general(EmdWarp<NW, T> *sw, int ncyc, int 
     return PILOT_ST_CONVERGED;
 }
 
-template <int NW, typename T>
+// PLAN (double only): problems from the pair list of `plan`, and each problem's plan written from its basis
+template <int NW, typename T, bool PLAN = false>
 __global__ void __launch_bounds__(EMD_WARPS * 32, 1)
 emd_pairs_kernel(const double *__restrict__ props, int K, const double *__restrict__ cost,
                  const unsigned short *__restrict__ arcs, int n_arcs_pad, PairMap pm, long long max_pivots,
                  double *__restrict__ out, int *__restrict__ status, int *__restrict__ pivots_out,
-                 unsigned long long *__restrict__ counter, int fast_limit, int scan_rows)
+                 unsigned long long *__restrict__ counter, int fast_limit, int scan_rows, PlanArgs<PLAN> plan)
 {
+    static_assert(!PLAN || sizeof(T) == sizeof(double), "plans are FP64 only");
     using W = EmdWarp<NW, T>;
     constexpr int KP = W::KP, NS = W::NS;
     constexpr int LDM = KP + 1;  // odd row stride
@@ -273,7 +275,19 @@ emd_pairs_kernel(const double *__restrict__ props, int K, const double *__restri
         l = __shfl_sync(FULLMASK, l, 0);
         if ((long long)l >= pm.n_local) break;
         int si_, sj_;
-        global_to_ij(pm, local_to_global(pm, (long long)l), si_, sj_);
+        if constexpr (PLAN) {
+            if (!plan_pair(plan, (long long)l, si_, sj_)) {
+                double *g = plan.plans + (long long)l * K * K;
+                for (int e = lane; e < K * K; e += 32) g[e] = __longlong_as_double(PILOT_NAN_BITS);
+                if (lane == 0) {
+                    out[l] = __longlong_as_double(PILOT_NAN_BITS);
+                    if (status) status[l] = PILOT_ST_NUMERIC;
+                }
+                continue;
+            }
+        } else {
+            global_to_ij(pm, local_to_global(pm, (long long)l), si_, sj_);
+        }
         const double *pa = props + (long long)si_ * K, *pb = props + (long long)sj_ * K;
 
         // ---------------- load a, b ; emd2's rescale of b ----------------
@@ -626,6 +640,18 @@ emd_pairs_kernel(const double *__restrict__ props, int K, const double *__restri
             }
         }
         acc = warp_sum_d(acc);
+        if constexpr (PLAN) {
+            // zero-fill, then the basis flows with the mapping of the objective loop: Gamma[row, column]
+            double *g = plan.plans + (long long)l * K * K;
+            for (int e = lane; e < K * K; e += 32) g[e] = 0.0;
+            __syncwarp();
+#pragma unroll
+            for (int s = 0; s < NS; ++s) {
+                const int y = s * 32 + lane;
+                const int p = sw->info[y] & 0xff;
+                if (p != 255) g[(s < NW) ? y * K + (p - KP) : p * K + (y - KP)] = (double)sw->flow[y];
+            }
+        }
         if (lane == 0) {
             out[l] = st == PILOT_ST_NUMERIC ? __longlong_as_double(0x7ff8000000000000LL) : acc;
             if (status) status[l] = st;
@@ -635,9 +661,10 @@ emd_pairs_kernel(const double *__restrict__ props, int K, const double *__restri
     }
 }
 
-template <int NW, typename T>
+template <int NW, typename T, bool PLAN = false>
 static int emd_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
-                      double *out, int *status, int *pivots, void *workspace, cudaStream_t st)
+                      double *out, int *status, int *pivots, void *workspace, cudaStream_t st,
+                      const PlanArgs<PLAN> &plan = {})
 {
     using W = EmdWarp<NW, T>;
     unsigned long long *counter = (unsigned long long *)workspace;
@@ -646,7 +673,8 @@ static int emd_launch(const double *props, int K, const double *cost, const Pair
     emd_sort_arcs_kernel<<<1, 1024, 0, st>>>(cost, K, n_arcs_pad, arcs);
     PILOT_LAUNCH_CHECK();
     const size_t smem = sizeof(T) * W::KP * (W::KP + 1) + sizeof(unsigned short) * n_arcs_pad + sizeof(W) * EMD_WARPS;
-    PILOT_CUDA(cudaFuncSetAttribute(emd_pairs_kernel<NW, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PILOT_CUDA(cudaFuncSetAttribute(emd_pairs_kernel<NW, T, PLAN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)smem));
     long long ctas = sm_count();
     const long long need = (pm.n_local + EMD_WARPS - 1) / EMD_WARPS;
     if (ctas > need) ctas = need;
@@ -665,14 +693,16 @@ static int emd_launch(const double *props, int K, const double *cost, const Pair
         if (scan_rows < 1) scan_rows = 1;
         if (scan_rows > K) scan_rows = K;
     }
-    emd_pairs_kernel<NW, T><<<(unsigned)ctas, EMD_WARPS * 32, smem, st>>>(
-        props, K, cost, arcs, n_arcs_pad, pm, max_pivots, out, status, pivots, counter, fast_limit, scan_rows);
+    emd_pairs_kernel<NW, T, PLAN><<<(unsigned)ctas, EMD_WARPS * 32, smem, st>>>(
+        props, K, cost, arcs, n_arcs_pad, pm, max_pivots, out, status, pivots, counter, fast_limit, scan_rows, plan);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
 
 int emd_general_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
                        double *out, int *status, int *pivots, void *workspace, cudaStream_t st);
+int emd_general_plans_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
+                             double *out, int *status, void *workspace, const PlanArgs<true> &plan, cudaStream_t st);
 
 size_t emd_ws_bytes(int K)
 {
@@ -707,4 +737,26 @@ extern "C" int pilot_emd_pairs(const double *props, int S, int K, const double *
     }
     if (K <= 32) return emd_launch<1, float>(props, K, cost, pm, max_pivots, out, status, pivots, workspace, st);
     return emd_launch<2, float>(props, K, cost, pm, max_pivots, out, status, pivots, workspace, st);
+}
+
+extern "C" int pilot_emd_plans(const double *props, int S, int K, const double *cost, int64_t max_pivots,
+                               const int32_t *pair_a, const int32_t *pair_b, int64_t n, double *plans, double *out,
+                               int32_t *status, void *workspace, size_t workspace_bytes, void *stream)
+{
+    using namespace pilot;
+    PILOT_CHECK_ARG(props && cost && pair_a && pair_b && plans && out && workspace, "pilot_emd_plans: NULL pointer");
+    PILOT_CHECK_ARG(S >= 1, "pilot_emd_plans: S=%d", S);
+    PILOT_CHECK_ARG(K >= 1 && K <= 256, "pilot_emd_plans: K=%d outside the supported range [1, 256]", K);
+    PILOT_CHECK_ARG(n >= 0, "pilot_emd_plans: n=%lld", (long long)n);
+    PILOT_CHECK_ARG(workspace_bytes >= emd_ws_bytes(K), "pilot_emd_plans: workspace too small");
+    if (n == 0) return 0;
+    if (max_pivots <= 0) max_pivots = 100000;  // POT numItermax default
+    const PairMap pm = plan_pair_map(n, S);
+    const PlanArgs<true> plan{pair_a, pair_b, S, plans};
+    cudaStream_t st = (cudaStream_t)stream;
+    PILOT_CUDA(cudaMemsetAsync(workspace, 0, 256, st));
+    if (K > 64) return emd_general_plans_launch(props, K, cost, pm, max_pivots, out, status, workspace, plan, st);
+    if (K <= 32)
+        return emd_launch<1, double, true>(props, K, cost, pm, max_pivots, out, status, nullptr, workspace, st, plan);
+    return emd_launch<2, double, true>(props, K, cost, pm, max_pivots, out, status, nullptr, workspace, st, plan);
 }

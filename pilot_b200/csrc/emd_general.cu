@@ -35,11 +35,13 @@ __host__ __device__ __forceinline__ size_t emg_state_bytes(int K)
     return ((N * (8 + 8 + 2 + 2 + 1)) + 15) & ~(size_t)15;
 }
 
+// PLAN: problems from the pair list of `plan`, and each problem's plan written from the real tree arcs
+template <bool PLAN>
 __global__ void __launch_bounds__(512)
 emd_general_kernel(const double *__restrict__ props, int K, const double *__restrict__ cost, PairMap pm,
                    long long max_pivots, double *__restrict__ out, int *__restrict__ status,
                    int *__restrict__ pivots_out, unsigned long long *__restrict__ counter,
-                   const double *__restrict__ art_p)
+                   const double *__restrict__ art_p, PlanArgs<PLAN> plan)
 {
     const double art = *art_p;  // big-M cost of the artificial arcs (emg_art_kernel)
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -60,7 +62,19 @@ emd_general_kernel(const double *__restrict__ props, int K, const double *__rest
         l = __shfl_sync(0xffffffffu, l, 0);
         if ((long long)l >= pm.n_local) break;
         int si, sj;
-        global_to_ij(pm, local_to_global(pm, (long long)l), si, sj);
+        if constexpr (PLAN) {
+            if (!plan_pair(plan, (long long)l, si, sj)) {
+                double *g = plan.plans + (long long)l * K * K;
+                for (int e = lane; e < K * K; e += 32) g[e] = __longlong_as_double(PILOT_NAN_BITS);
+                if (lane == 0) {
+                    out[l] = __longlong_as_double(PILOT_NAN_BITS);
+                    if (status) status[l] = PILOT_ST_NUMERIC;
+                }
+                continue;
+            }
+        } else {
+            global_to_ij(pm, local_to_global(pm, (long long)l), si, sj);
+        }
         const double *pa = props + (long long)si * K, *pb = props + (long long)sj * K;
 
         // ---- a, b (emd2 rescales b to the mass of a), the artificial star ----
@@ -193,6 +207,17 @@ emd_general_kernel(const double *__restrict__ props, int K, const double *__rest
         }
         acc = warp_sum_d(acc);
         infeasible = __any_sync(0xffffffffu, infeasible);
+        if constexpr (PLAN) {
+            // zero-fill, then the flows of the real tree arcs with the mapping of the cost loop
+            double *g = plan.plans + (long long)l * K * K;
+            for (int e = lane; e < K * K; e += 32) g[e] = 0.0;
+            __syncwarp();
+            for (int u = lane; u < root; u += 32) {
+                const int p = s.parent[u];
+                if (p == root) continue;
+                g[u < K ? (long long)u * K + (p - K) : (long long)p * K + (u - K)] = s.flow[u];
+            }
+        }
         if (lane == 0) {
             const bool bad = !(sa == sa) || !(sb == sb) || (st == PILOT_ST_CONVERGED && infeasible);
             out[l] = bad ? __longlong_as_double(0x7ff8000000000000LL) : acc;
@@ -219,8 +244,10 @@ __global__ void emg_art_kernel(const double *__restrict__ cost, int K, double *_
     }
 }
 
-int emd_general_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
-                       double *out, int *status, int *pivots, void *workspace, cudaStream_t st)
+template <bool PLAN>
+static int emg_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
+                      double *out, int *status, int *pivots, void *workspace, const PlanArgs<PLAN> &plan,
+                      cudaStream_t st)
 {
     unsigned long long *counter = (unsigned long long *)workspace;
     double *art = (double *)((char *)workspace + 128);
@@ -231,15 +258,28 @@ int emd_general_launch(const double *props, int K, const double *cost, const Pai
     if (warps > 16) warps = 16;
     if (warps < 1) warps = 1;
     const size_t smem = per_warp * warps;
-    PILOT_CUDA(cudaFuncSetAttribute(emd_general_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PILOT_CUDA(cudaFuncSetAttribute(emd_general_kernel<PLAN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)smem));
     long long ctas = sm_count();
     const long long need = (pm.n_local + warps - 1) / warps;
     if (ctas > need) ctas = need;
     if (ctas < 1) ctas = 1;
-    emd_general_kernel<<<(unsigned)ctas, warps * 32, smem, st>>>(props, K, cost, pm, max_pivots, out, status, pivots,
-                                                                counter, art);
+    emd_general_kernel<PLAN><<<(unsigned)ctas, warps * 32, smem, st>>>(props, K, cost, pm, max_pivots, out, status,
+                                                                      pivots, counter, art, plan);
     PILOT_LAUNCH_CHECK();
     return 0;
+}
+
+int emd_general_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
+                       double *out, int *status, int *pivots, void *workspace, cudaStream_t st)
+{
+    return emg_launch<false>(props, K, cost, pm, max_pivots, out, status, pivots, workspace, {}, st);
+}
+
+int emd_general_plans_launch(const double *props, int K, const double *cost, const PairMap &pm, long long max_pivots,
+                             double *out, int *status, void *workspace, const PlanArgs<true> &plan, cudaStream_t st)
+{
+    return emg_launch<true>(props, K, cost, pm, max_pivots, out, status, nullptr, workspace, plan, st);
 }
 
 }  // namespace pilot

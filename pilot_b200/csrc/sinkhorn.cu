@@ -149,3 +149,30 @@ extern "C" int pilot_sinkhorn_pairs(const double *props, int S, int K, const dou
     // problems the scaled form could not represent (normally none): reference-form kernel
     return sinkhorn_ref_launch(props, K, cost, prm, pm, res, redo_cap, &ws.ctr->slow, ws.gibbs, st);
 }
+
+extern "C" int pilot_sinkhorn_plans(const double *props, int S, int K, const double *cost, double reg,
+                                    int num_iter_max, double stop_thr, double tau, int check_every,
+                                    const int32_t *pair_a, const int32_t *pair_b, int64_t n, double *plans,
+                                    double *out, int32_t *iters, int32_t *absorptions, int32_t *status,
+                                    void *workspace, size_t workspace_bytes, void *stream)
+{
+    using namespace pilot;
+    PILOT_CHECK_ARG(props && cost && pair_a && pair_b && plans && out && workspace,
+                    "pilot_sinkhorn_plans: NULL pointer");
+    PILOT_CHECK_ARG(S >= 1, "pilot_sinkhorn_plans: S=%d", S);
+    PILOT_CHECK_ARG(K >= 1 && K <= 256, "pilot_sinkhorn_plans: K=%d outside the supported range [1, 256]", K);
+    PILOT_CHECK_ARG(n >= 0, "pilot_sinkhorn_plans: n=%lld", (long long)n);
+    PILOT_CHECK_ARG(reg > 0.0, "pilot_sinkhorn_plans: reg must be > 0");
+    PILOT_CHECK_ARG(num_iter_max >= 1 && check_every >= 1, "pilot_sinkhorn_plans: bad iteration parameters");
+    const SkWorkspace ws = sk_workspace(workspace, K);
+    PILOT_CHECK_ARG(workspace_bytes >= ws.bytes, "pilot_sinkhorn_plans: workspace %zu < %zu bytes", workspace_bytes,
+                    ws.bytes);
+    if (n == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    const SkParams prm{reg, stop_thr, tau, num_iter_max, check_every};
+    const SkOut res{out, iters, absorptions, status, ws.redo, &ws.ctr->n_redo};
+    PILOT_CUDA(cudaMemsetAsync(ws.ctr, 0, sizeof(SkCounters), st));
+    // the reference form: POT's own statement of Gamma, for every K <= 256 (bit-identical costs to algo = 1)
+    return sinkhorn_ref_plans_launch(props, K, cost, prm, plan_pair_map(n, S), res,
+                                     PlanArgs<true>{pair_a, pair_b, S, plans}, &ws.ctr->slow, ws.gibbs, st);
+}

@@ -110,6 +110,10 @@ constexpr long long SK_SOLVE_ALL = -1;
 int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
                         const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
                         cudaStream_t st);
+// plan variant (pilot_sinkhorn_plans): mode 0 over the pair list of `plan`, pm = plan_pair_map(n, S)
+int sinkhorn_ref_plans_launch(const double *props, int K, const double *cost, const SkParams &prm,
+                              const PairMap &pm, const SkOut &res, const PlanArgs<true> &plan,
+                              unsigned long long *counter, double *gibbs, cudaStream_t st);
 
 int skb_pad(int K);
 // storage extent of the setup buffer: skb_pad(K) up to 64 types, roundup(K, 8) above

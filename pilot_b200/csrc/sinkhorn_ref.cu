@@ -49,13 +49,16 @@ __device__ __forceinline__ double block_sum64(double v, double *red)
 // more than max_list problems were queued (the list overflowed): scan out[] for the redo marker the fast
 // kernels left behind and solve those (the listed ones were overwritten by mode 1 already).
 // GK: the Gibbs matrix lives in the CTA's slice of `gibbs` (K x (K | 1) doubles) instead of shared memory.
-template <bool GK>
+// PLAN (mode 0 only): problems from the pair list of `plan`; thread t writes column t of Gamma in the loop that
+// accumulates the cost, so the plan sums, in that order, to out[l].
+template <bool GK, bool PLAN = false>
 __global__ void __launch_bounds__(SKR_MAX_WARPS * 32)
 sinkhorn_ref_kernel(const double *__restrict__ props, int K, const double *__restrict__ M, SkParams prm,
                     PairMap pm, int mode, const long long *__restrict__ list,
                     const unsigned long long *__restrict__ n_list_dev, long long max_list,
                     double *__restrict__ out, int *__restrict__ iters_out, int *__restrict__ abs_out,
-                    int *__restrict__ status_out, unsigned long long *__restrict__ counter, double *gibbs)
+                    int *__restrict__ status_out, unsigned long long *__restrict__ counter, double *gibbs,
+                    PlanArgs<PLAN> plan)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int KS = K | 1;  // odd row stride: row- and column-walks are both conflict-free
@@ -109,7 +112,21 @@ sinkhorn_ref_kernel(const double *__restrict__ props, int K, const double *__res
             l = mode == 1 ? list[w] : w;
         }
         int si, sj;
-        global_to_ij(pm, local_to_global(pm, l), si, sj);
+        if constexpr (PLAN) {
+            if (!plan_pair(plan, l, si, sj)) {
+                double *g = plan.plans + l * K * K;
+                for (int e = t; e < K * K; e += NT) g[e] = __longlong_as_double(PILOT_NAN_BITS);
+                if (t == 0) {
+                    out[l] = __longlong_as_double(PILOT_NAN_BITS);
+                    if (iters_out) iters_out[l] = 0;
+                    if (abs_out) abs_out[l] = 0;
+                    if (status_out) status_out[l] = PILOT_ST_NUMERIC;
+                }
+                continue;
+            }
+        } else {
+            global_to_ij(pm, local_to_global(pm, l), si, sj);
+        }
         const double a = act ? props[(long long)si * K + t] : 0.0;
         const double b = act ? props[(long long)sj * K + t] : 0.0;
         if (act) { al[t] = 0.0; be[t] = 0.0; u[t] = 1.0 / K; v[t] = 1.0 / K; }
@@ -188,7 +205,9 @@ sinkhorn_ref_kernel(const double *__restrict__ props, int K, const double *__res
             const double bj = be[t], lvj = lv[t];
             for (int i = 0; i < K; ++i) {
                 const double m = __ldg(M + i * K + t);
-                c += m * exp(-(m - al[i] - bj) / reg + lu[i] + lvj);
+                const double g = exp(-(m - al[i] - bj) / reg + lu[i] + lvj);
+                if constexpr (PLAN) plan.plans[l * K * K + i * K + t] = g;
+                c += m * g;
             }
         }
         c = block_sum64(c, red);
@@ -212,9 +231,10 @@ size_t sinkhorn_ref_gibbs_bytes(int K)
     return skr_global_gibbs(K) ? sizeof(double) * (size_t)sm_count() * K * (K | 1) : 0;
 }
 
-int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
-                        const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
-                        cudaStream_t st)
+template <bool PLAN>
+static int skr_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
+                      const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
+                      const PlanArgs<PLAN> &plan, cudaStream_t st)
 {
     const bool queued = redo_cap != SK_SOLVE_ALL;
     // with a device-side list the amount of work is unknown here: launch one wave and let the CTAs loop
@@ -225,7 +245,7 @@ int sinkhorn_ref_launch(const double *props, int K, const double *cost, const Sk
     const size_t smem = gk ? sizeof(double) * (8 * (size_t)K + SKR_MAX_WARPS) : sinkhorn_ref_smem(K);
     const int threads = skr_threads(K);
     PILOT_CHECK_ARG(threads <= SKR_MAX_WARPS * 32, "sinkhorn reference-form kernel: K=%d too large", K);
-    const auto kern = gk ? sinkhorn_ref_kernel<true> : sinkhorn_ref_kernel<false>;
+    const auto kern = gk ? sinkhorn_ref_kernel<true, PLAN> : sinkhorn_ref_kernel<false, PLAN>;
     PILOT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
     PILOT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
@@ -236,10 +256,25 @@ int sinkhorn_ref_launch(const double *props, int K, const double *cost, const Sk
     for (int mode = queued ? 1 : 0; mode <= (queued ? 2 : 0); ++mode) {
         PILOT_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
         kern<<<(unsigned)ctas, threads, smem, st>>>(props, K, cost, prm, pm, mode, res.redo, res.n_redo, redo_cap,
-                                                    res.out, res.iters, res.absn, res.status, counter, gibbs);
+                                                    res.out, res.iters, res.absn, res.status, counter, gibbs,
+                                                    plan);
         PILOT_LAUNCH_CHECK();
     }
     return 0;
+}
+
+int sinkhorn_ref_launch(const double *props, int K, const double *cost, const SkParams &prm, const PairMap &pm,
+                        const SkOut &res, long long redo_cap, unsigned long long *counter, double *gibbs,
+                        cudaStream_t st)
+{
+    return skr_launch<false>(props, K, cost, prm, pm, res, redo_cap, counter, gibbs, {}, st);
+}
+
+int sinkhorn_ref_plans_launch(const double *props, int K, const double *cost, const SkParams &prm,
+                              const PairMap &pm, const SkOut &res, const PlanArgs<true> &plan,
+                              unsigned long long *counter, double *gibbs, cudaStream_t st)
+{
+    return skr_launch<true>(props, K, cost, prm, pm, res, SK_SOLVE_ALL, counter, gibbs, plan, st);
 }
 
 }  // namespace pilot

@@ -199,6 +199,61 @@ def emd_pairs(props: torch.Tensor, cost: torch.Tensor, rng: PairRange, max_pivot
     return out[:n]
 
 
+def _plan_inputs(props: torch.Tensor, cost: torch.Tensor, pair_a, pair_b):
+    """Checked shapes and int32 device copies of the pair lists (a list, an ndarray or a tensor)."""
+    _require_cuda(props, cost)
+    assert props.dtype == torch.float64 and cost.dtype == torch.float64
+    assert props.is_contiguous() and cost.is_contiguous()
+    S, K = props.shape
+    assert cost.shape == (K, K)
+    dev = props.device
+    pa, pb = (torch.as_tensor(p, dtype=torch.int32).to(dev).contiguous().reshape(-1) for p in (pair_a, pair_b))
+    if pa.numel() != pb.numel():
+        raise ValueError(f"pair_a has {pa.numel()} entries and pair_b {pb.numel()}")
+    n = pa.numel()
+    plans = torch.empty((n, K, K), dtype=torch.float64, device=dev)
+    out = torch.empty((n,), dtype=torch.float64, device=dev)
+    return S, K, n, pa, pb, plans, out
+
+
+def emd_plans(props: torch.Tensor, cost: torch.Tensor, pair_a, pair_b, max_pivots: int = 100000,
+              want_info: bool = False):
+    """Exact-EMD transport plans of the problems (props[pair_a[l]], props[pair_b[l]]), FP64, no mirroring:
+    (plans [n, K, K], out [n]) with plans[l, r, c] the mass moved from type r of a to type c of b (emd2's rescaled
+    b) and out[l] the cost pilot_emd_pairs computes for that pair; with want_info also status [n].  A pair index
+    outside [0, S) gives a NaN plan, a NaN cost and ST_NUMERIC."""
+    S, K, n, pa, pb, plans, out = _plan_inputs(props, cost, pair_a, pair_b)
+    status = torch.zeros((n,), dtype=torch.int32, device=props.device) if want_info else None
+    ws = _workspace(lib().pilot_workspace_bytes(_lib.WS_EMD, n, K, S, 0), props.device)
+    check(lib().pilot_emd_plans(_ptr(props), S, K, _ptr(cost), int(max_pivots), _ptr(pa), _ptr(pb), n, _ptr(plans),
+                                _ptr(out), _ptr(status), _ptr(ws), ws.numel(), _stream()), "pilot_emd_plans")
+    if want_info:
+        return plans, out, status
+    return plans, out
+
+
+def sinkhorn_plans(props: torch.Tensor, cost: torch.Tensor, reg: float, pair_a, pair_b, num_iter_max: int = 1000,
+                   stop_thr: float = 1e-9, tau: float = 1e3, check_every: int = 20, want_info: bool = False):
+    """Stabilised-Sinkhorn transport plans of the problems (props[pair_a[l]], props[pair_b[l]]), FP64, in POT's
+    reference form: (plans [n, K, K], out [n]), out bit-identical to sinkhorn_pairs(algo=1) for the same pair; with
+    want_info also (iters, absorptions, status) [n] each.  A pair index outside [0, S) gives a NaN plan, a NaN
+    cost and ST_NUMERIC."""
+    S, K, n, pa, pb, plans, out = _plan_inputs(props, cost, pair_a, pair_b)
+    iters = absn = status = None
+    if want_info:
+        iters = torch.zeros((n,), dtype=torch.int32, device=props.device)
+        absn = torch.zeros_like(iters)
+        status = torch.zeros_like(iters)
+    ws = _workspace(lib().pilot_workspace_bytes(_lib.WS_SINKHORN, n, K, S, 0), props.device)
+    check(lib().pilot_sinkhorn_plans(_ptr(props), S, K, _ptr(cost), float(reg), int(num_iter_max), float(stop_thr),
+                                     float(tau), int(check_every), _ptr(pa), _ptr(pb), n, _ptr(plans), _ptr(out),
+                                     _ptr(iters), _ptr(absn), _ptr(status), _ptr(ws), ws.numel(), _stream()),
+          "pilot_sinkhorn_plans")
+    if want_info:
+        return plans, out, iters, absn, status
+    return plans, out
+
+
 def unpack_pairs(packed: torch.Tensor, chunk_stride: int, S: int, rng: PairRange, diag_value: float = 0.0,
                  dense: Optional[torch.Tensor] = None) -> torch.Tensor:
     """All-gathered packed chunks -> dense float64 matrix: S x S, or S_a x (S - S_a) for PAIRS_RECT."""

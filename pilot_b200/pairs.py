@@ -157,6 +157,56 @@ def _mode_for(regularized, cost_norm, symmetric: Optional[bool], rect: bool = Fa
     return False, _lib.PAIRS_FULL  # Sinkhorn is neither symmetric nor zero on the diagonal (SURVEY fact 6)
 
 
+def plan_rule(rows, cols, S: int, mirrored: bool) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+    """Which problem produced each entry (rows[l], cols[l]) of a matrix: (pair_a, pair_b, transpose, diagonal).
+    Without mirroring the entry is the problem (i, j).  A mirrored matrix (exact EMD, symmetric metric-like cost)
+    holds (i, j) for i < j, the transpose of (j, i) for i > j, and an exact 0 on the diagonal: there the plan is
+    diag(props[i]), which is optimal for a symmetric, non-negative, zero-diagonal cost, and nothing is solved.
+    An index outside [0, S) is passed through, so that the solver reports it (NaN)."""
+    i = np.asarray(rows, dtype=np.int64).reshape(-1)
+    j = np.asarray(cols, dtype=np.int64).reshape(-1)
+    if i.shape != j.shape:
+        raise ValueError(f"{i.size} row indices and {j.size} column indices")
+    if not mirrored:
+        none = np.zeros(i.shape, dtype=bool)
+        return i, j, none, none
+    flip = i > j
+    diag = (i == j) & (i >= 0) & (i < S)
+    return np.where(flip, j, i), np.where(flip, i, j), flip, diag
+
+
+def entry_plans(props: torch.Tensor, cost_norm: torch.Tensor, rows, cols, regularized="unreg", reg: float = 0.1,
+                symmetric: Optional[bool] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Transport plans behind the entries (rows[l], cols[l]) of ``all_pairs(props, cost_norm, regularized, reg,
+    symmetric=symmetric)``: (plans [n, K, K], costs [n]) on the device, plans[l, r, c] the mass that row sample's
+    type r sends to column sample's type c.  Each plan is that of the problem that produced the entry (plan_rule),
+    so an exact-EMD cost equals the matrix entry bit for bit; a Sinkhorn plan comes from the reference form
+    (ops.sinkhorn_plans), within 1e-12 relative of the entry."""
+    S, K = props.shape
+    exact, mode = _mode_for(regularized, cost_norm, symmetric)
+    pa, pb, flip, diag = plan_rule(rows, cols, S, exact and mode == _lib.PAIRS_UPPER)
+    n = pa.size
+    dev = props.device
+    plans = torch.empty((n, K, K), dtype=torch.float64, device=dev)
+    costs = torch.empty((n,), dtype=torch.float64, device=dev)
+    solve = np.nonzero(~diag)[0]
+    if solve.size:
+        if exact:
+            g, c = ops.emd_plans(props, cost_norm, pa[solve], pb[solve])
+        else:
+            g, c = ops.sinkhorn_plans(props, cost_norm, reg, pa[solve], pb[solve])
+        f = torch.from_numpy(flip[solve]).to(dev).view(-1, 1, 1)
+        sel = torch.from_numpy(solve).to(dev)
+        plans[sel] = torch.where(f, g.transpose(1, 2), g)
+        costs[sel] = c
+    d = np.nonzero(diag)[0]
+    if d.size:
+        sel = torch.from_numpy(d).to(dev)
+        plans[sel] = torch.diag_embed(props[torch.from_numpy(pa[d]).to(dev)])
+        costs[sel] = 0.0
+    return plans, costs
+
+
 def _solve_window(props, cost_norm, exact: bool, reg: float, mode: int, first: int, total: int, nranks: int,
                   rank: int, group, algo: int, precision, dense: torch.Tensor, want_info: bool = False,
                   marks: Optional[list] = None, rows: int = 0):

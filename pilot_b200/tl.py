@@ -24,6 +24,7 @@ import pandas as pd
 import torch
 
 from . import ops, pairs
+from . import pairs as _pairs  # wasserstein_plans takes an argument named `pairs`
 from .h5ad import load_h5ad  # noqa: F401  (pilotpy.tl.load_h5ad, Trajectory.py:121-137)
 
 warnings.filterwarnings("ignore")  # the reference silences everything at import (Trajectory.py:32)
@@ -625,6 +626,64 @@ def wasserstein_d_extend(Clu_rep, EMD, Clu_rep_new, cost, regularized="unreg", r
     out[:S_old, :S_old] = EMD
     # the square's frame takes its transpose; a mirrored matrix is its own transpose
     return out, _emd_frame(out, ids_old + ids_new, out.copy() if sym else None)
+
+
+_PLAN_CHUNK_BYTES = 256 << 20  # device memory of the plans of one chunk (512 plans at K = 256)
+
+
+def wasserstein_plans(Clu_rep, cost, pairs, regularized="unreg", reg=0.1, Clu_rep_b=None):
+    """Transport plans of chosen sample pairs: what the distance between two samples is made of.
+
+    ``pairs`` is a sequence of ``(id_a, id_b)``.  Without ``Clu_rep_b`` both ids are keys of ``Clu_rep`` and the
+    plans follow ``wasserstein_d(Clu_rep, cost, regularized, reg)``; with it ``id_a`` is a key of ``Clu_rep`` and
+    ``id_b`` of ``Clu_rep_b``, and they follow ``wasserstein_d_cross(Clu_rep, Clu_rep_b, ...)``.  Returns
+    ``(plans ndarray [n, K, K], costs ndarray [n])``: ``plans[l, r, c]`` is the mass that cell type r of id_a
+    sends to cell type c of id_b, and ``sum(cost * plans[l])`` is the distance.  Exact EMD
+    (``regularized == "unreg"``): ``costs`` equal the matrix entries bit for bit (a mirrored matrix gives the
+    transposed plan of (id_b, id_a), and ``diag(a)`` with cost 0 on its diagonal).  Sinkhorn: POT's reference form
+    of the plan, costs within 1e-12 relative of the matrix entries.  Solved on the GPU in FP64, in chunks."""
+    ids_a, P_a = _stack_props(Clu_rep)
+    ids_b, P_b = _stack_props(Clu_rep_b) if Clu_rep_b is not None else (ids_a, P_a)
+    pos_a = {s: i for i, s in enumerate(ids_a)}
+    pos_b = {s: i for i, s in enumerate(ids_b)}
+    rows = np.array([pos_a[a] for a, _ in pairs], dtype=np.int64)  # KeyError for an unknown id
+    cols = np.array([pos_b[b] for _, b in pairs], dtype=np.int64)
+    C = np.ascontiguousarray(np.asarray(cost, dtype=np.float64))
+    if rows.size == 0:
+        K = C.shape[0] if C.ndim == 2 else 0
+        return np.zeros((0, K, K)), np.zeros((0,))
+    _check_two_sets(P_a, P_b, C, regularized)
+    if Clu_rep_b is not None:  # the block between two sets never mirrors
+        P = np.concatenate([P_a, P_b])
+        cols = cols + len(ids_a)
+        sym = False
+    else:
+        P = P_a
+        sym = _pairs.cost_is_symmetric_metric_like(C) if regularized == "unreg" else None
+    K = C.shape[0]
+    n = rows.size
+    plans = np.empty((n, K, K), dtype=np.float64)
+    costs = np.empty((n,), dtype=np.float64)
+    P_d, C_d = _to_device(np.ascontiguousarray(P)), _to_device(C)
+    chunk = max(1, _PLAN_CHUNK_BYTES // (8 * K * K))
+    for s in range(0, n, chunk):
+        g, c = _pairs.entry_plans(P_d, C_d, rows[s:s + chunk], cols[s:s + chunk], regularized, reg, symmetric=sym)
+        plans[s:s + chunk] = g.cpu().numpy()
+        costs[s:s + chunk] = c.cpu().numpy()
+    return plans, costs
+
+
+def transport_plan(adata, sample_a, sample_b, regularized="unreg", reg=0.1):
+    """The transport plan between two samples after ``wasserstein_distance``: ``(DataFrame K x K, cost)``, index =
+    the cell types of ``sample_a`` (the mass it sends), columns = those of ``sample_b``, both named as in
+    ``adata.uns['cost']``.  The cost is normalised as ``wasserstein_distance`` does (``cost / cost.max()``, the same
+    IEEE division), so with that call's ``regularized`` and ``reg`` an exact-EMD cost equals
+    ``adata.uns['EMD'][i, j]`` bit for bit."""
+    cost_df = adata.uns["cost"]
+    C = np.asarray(cost_df.to_numpy(), dtype=np.float64)
+    plans, costs = wasserstein_plans(adata.uns["proportions"], C / C.max(), [(sample_a, sample_b)], regularized, reg)
+    frame = pd.DataFrame(plans[0], index=cost_df.index.copy(), columns=cost_df.columns.copy())
+    return frame, float(costs[0])
 
 
 # ---------------------------------------------------------------------------
