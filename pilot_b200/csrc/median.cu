@@ -3,8 +3,8 @@
 // (reference pilotpy/tools/Trajectory.py:465-466; pandas nanmedian semantics:
 // NaNs ignored, even counts -> (lo + hi) / 2 rounded in the input dtype).
 //
-// Two exact paths:
-//  * sampled-pivot streaming path (default for n >= 64K; second half of this file):
+// Two exact paths, chosen by median_path (end of this file):
+//  * sampled-pivot streaming path (n >= 64K rows; second half of this file):
 //    a hashed sample of ~2048-4096 rows per type gives, per (type, dim), two pivots lo <= hi that bracket the
 //    median with ~4e-8 failure odds; ONE pass over X then counts x < lo and collects the ~10 % of elements
 //    inside the bracket in per-pair lists (mn_stream_run_kernel: a CTA counting-sorts the row ids of a chunk
@@ -13,7 +13,8 @@
 //    outside its bracket (or its list overflows) the same CTA falls back to an exact radix select over
 //    the type's rows -- no host round trip, results are always exact.
 //    HBM traffic: one read of X + ~6 % for the sample + the lists (written once, read once).
-//  * most-significant-digit radix select (small inputs, huge K*D): every pass streams X once
+//  * most-significant-digit radix select (every other input: fewer rows, a large K*D, more types than the stream
+//    pass's shared memory holds, rows 1 MiB or more apart): every pass streams X once
 //    and histograms the current 8-bit digit of the elements whose higher digits match the
 //    running prefix of their (type, dim) query; 4 passes for f32, 8 for f64.
 // Two queries per (type, dim) (ranks (n-1)/2 and n/2) so even counts need no second selection.
@@ -54,20 +55,32 @@ template <> struct KeyOf<double> {
     }
 };
 
-// workspace layout (all 8-byte aligned):
-//   hist   : KD * 2 * 256 u32
-//   prefix : KD * 2 key (stored as u64)
-//   rank   : KD * 2 u64
-//   nvalid : KD u64
 struct MedianWs {
-    unsigned int *hist;
-    unsigned long long *prefix, *rank, *nvalid;
+    unsigned int *hist;                          // KD * 2 * 256
+    unsigned long long *prefix, *rank, *nvalid;  // KD * 2 keys (stored as u64), KD * 2, KD
 };
 
-static size_t median_ws_bytes_impl(int K, int D)
+// the radix path's workspace (all 8-byte aligned)
+struct MedianLayout {
+    MedianWs ws;
+    size_t hist_bytes;  // zeroed before every pass
+    size_t bytes;       // end of the last region
+};
+
+// carves the radix path's workspace at `base` (nullptr: only its size)
+static MedianLayout median_workspace(void *base, int K, int D)
 {
-    size_t kd = (size_t)K * D;
-    return kd * 2 * 256 * sizeof(unsigned int) + kd * 2 * 8 + kd * 2 * 8 + kd * 8;
+    const size_t kd = (size_t)K * D;
+    uintptr_t p = (uintptr_t)base;
+    const auto take = [&p](size_t bytes) { const uintptr_t r = p; p += bytes; return r; };
+    MedianLayout l;
+    l.hist_bytes = kd * 2 * 256 * sizeof(unsigned int);
+    l.ws.hist = (unsigned int *)take(l.hist_bytes);
+    l.ws.prefix = (unsigned long long *)take(kd * 2 * 8);
+    l.ws.rank = (unsigned long long *)take(kd * 2 * 8);
+    l.ws.nvalid = (unsigned long long *)take(kd * 8);
+    l.bytes = p - (uintptr_t)base;
+    return l;
 }
 
 template <typename T, int PASS>
@@ -206,21 +219,14 @@ static int median_run(const T *X, long long n, int D, long long ldx, const int *
                       double *cent64, void *workspace, cudaStream_t st)
 {
     const size_t kd = (size_t)K * D;
-    MedianWs ws;
-    unsigned char *p = (unsigned char *)workspace;
-    ws.hist = (unsigned int *)p;
-    const size_t hist_bytes = kd * 2 * 256 * sizeof(unsigned int);
-    p += hist_bytes;
-    ws.prefix = (unsigned long long *)p; p += kd * 2 * 8;
-    ws.rank = (unsigned long long *)p;   p += kd * 2 * 8;
-    ws.nvalid = (unsigned long long *)p;
+    const MedianLayout l = median_workspace(workspace, K, D);
     int rc;
 #define PILOT_MEDIAN_PASS(P) \
-    if (KeyOf<T>::PASSES > P) { rc = median_pass<T, (P < KeyOf<T>::PASSES ? P : 0)>(X, n, D, ldx, code, K, ws, hist_bytes, st); if (rc) return rc; }
+    if (KeyOf<T>::PASSES > P) { rc = median_pass<T, (P < KeyOf<T>::PASSES ? P : 0)>(X, n, D, ldx, code, K, l.ws, l.hist_bytes, st); if (rc) return rc; }
     PILOT_MEDIAN_PASS(0) PILOT_MEDIAN_PASS(1) PILOT_MEDIAN_PASS(2) PILOT_MEDIAN_PASS(3)
     PILOT_MEDIAN_PASS(4) PILOT_MEDIAN_PASS(5) PILOT_MEDIAN_PASS(6) PILOT_MEDIAN_PASS(7)
 #undef PILOT_MEDIAN_PASS
-    median_final_kernel<T><<<(unsigned)((kd + 127) / 128), 128, 0, st>>>((int)kd, ws, cent, cent64);
+    median_final_kernel<T><<<(unsigned)((kd + 127) / 128), 128, 0, st>>>((int)kd, l.ws, cent, cent64);
     PILOT_LAUNCH_CHECK();
     return 0;
 }
@@ -250,11 +256,9 @@ constexpr int MN_SAMPLE_MIN = 2048;     // target sample rows per type: n_k / 16
 constexpr int MN_SAMPLE_MAX = 4096;     //   (bracket width ~ 5.5 / sqrt(sample): 12 % ... 9 % of the type's values; measured best of 2048/4096/8192)
 constexpr int MN_MCAP = MN_SAMPLE_MAX + MN_SAMPLE_MAX / 4;  // most sample rows a type can hold (pivot kernel's buffer)
 constexpr double MED_SIGMAS = 5.5;      // half-width of the bracket in binomial sigmas
-constexpr int MN_THREADS = 512;         // stream kernel
 constexpr int MN_FIN_THREADS = 256;
 constexpr int MN_REP = 32;              // replicas of every (type, dim) list: same-address global atomics serialise at ~20 ns
 constexpr int MN_STAGE_MIN = 16384, MN_STAGE_MAX = 98304;  // bytes of candidates the finish kernel stages in shared memory
-constexpr size_t MN_SMEM_MAX = 160 * 1024;  // pivots + counters of every (type, dim) must fit
 
 // shared-memory reduction without the compiler's warp-aggregation collective
 __device__ __forceinline__ void red_shared_inc(unsigned int *p)
@@ -341,9 +345,6 @@ template <typename T> __global__ void mn_plan_kernel(int K, int D, int samp_max,
         off += __shfl_sync(0xffffffffu, ic, 31);
     }
 }
-
-// replica of a row's candidate lists: consecutive rows take consecutive replicas, with two folds against periods
-__device__ __forceinline__ unsigned mn_rep(unsigned row) { return (row + (row >> 5) + (row >> 10)) & (MN_REP - 1); }
 
 __device__ __forceinline__ unsigned mn_hash(unsigned i)
 {
@@ -573,13 +574,33 @@ __device__ bool cta_select2_linear(Src src, long long r0, long long r1, T vlo, T
     return true;
 }
 
+// CTA-level selection of the ranks r0 <= r1 among the values of `src` (no NaN), all of which lie in [vlo, vhi]: the
+// linear bins when the interval is finite and not a point; otherwise, or on a plateau of ties, the radix select from
+// the first digit in which key(vlo) and key(vhi) differ (every value shares the digits above it).
+template <typename T, typename Src>
+__device__ void cta_select2(Src src, long long r0, long long r1, T vlo, T vhi, unsigned int *hist /*[MN_LIN_BINS]*/,
+                            T *coll /*[MN_LIN_CAP + 2]*/, unsigned int *lsh /*[16]*/, long long *sh /*[4]*/, T &out0,
+                            T &out1)
+{
+    using KO = KeyOf<T>;
+    using Key = typename KO::type;
+    constexpr int BITS = sizeof(Key) * 8;
+    if (vlo < vhi && vhi - vlo < Inf<T>::pos() &&
+        cta_select2_linear<T>(src, r0, r1, vlo, vhi, hist, coll, lsh, out0, out1))
+        return;
+    const Key kl = KO::key(vlo), kh = KO::key(vhi);
+    int first = BITS - 8;
+    while (first > 0 && (kl >> first) == (kh >> first)) first -= 8;
+    const Key prefix = first < BITS - 8 ? (Key)((kl >> (first + 8)) << (first + 8)) : (Key)0;
+    cta_select2_raw<T>(src, r0, r1, hist, sh, prefix, first, out0, out1);
+}
+
 // one CTA per (type, dim): pivots lo <= hi bracketing the median, from the type's sample rows
 template <typename T>
 __global__ void __launch_bounds__(256, 6)
 mn_pivot_kernel(int D, MnWs<T> ws)
 {
-    using KO = KeyOf<T>;
-    using Key = typename KO::type;
+    using Key = typename KeyOf<T>::type;
     constexpr int BITS = sizeof(Key) * 8;
     __shared__ long long sh[4];
     __shared__ unsigned int lhist[MN_LIN_BINS], lsh[16];
@@ -629,11 +650,8 @@ mn_pivot_kernel(int D, MnWs<T> ws)
                 }
             };
             if (jhi < m) {  // both ranks fall on valid samples; otherwise the bracket stays open (hi = +inf)
-                bool done = false;
-                if (mn == mx) { lo = hi = mn; done = true; }
-                else if (mx - mn < Inf<T>::pos())
-                    done = cta_select2_linear<T>(smp, jlo, jhi, mn, mx, lhist, lcoll, lsh, lo, hi);
-                if (!done) cta_select2_raw<T>(smp, jlo, jhi, hist, sh, (Key)0, BITS - 8, lo, hi);
+                if (mn == mx) lo = hi = mn;
+                else cta_select2<T>(smp, jlo, jhi, mn, mx, lhist, lcoll, lsh, sh, lo, hi);
             } else if (jlo < m) {
                 T dummy;
                 cta_select2_raw<T>(smp, jlo, jlo, hist, sh, (Key)0, BITS - 8, lo, dummy);
@@ -646,98 +664,23 @@ mn_pivot_kernel(int D, MnWs<T> ws)
     }
 }
 
-// The streaming pass: X once, in memory order.
-template <typename T>
-__global__ void __launch_bounds__(MN_THREADS)
-mn_stream_kernel(const T *__restrict__ X, long long n, int D, long long ldx, const int *__restrict__ code, int K,
-                 MnWs<T> ws)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int KD = K * D;
-    T *spiv = reinterpret_cast<T *>(smem_raw);                                  // [KD][2]
-    unsigned long long *scoff = reinterpret_cast<unsigned long long *>(spiv + 2 * (size_t)KD);  // [K]
-    unsigned int *sbelow = reinterpret_cast<unsigned int *>(scoff + K);         // [KD]
-    unsigned int *sabove = sbelow + KD;                                         // [KD]
-    unsigned int *scap = sabove + KD;                                           // [K]
-    for (int i = threadIdx.x; i < 2 * KD; i += blockDim.x) spiv[i] = ws.piv[i];
-    for (int i = threadIdx.x; i < KD; i += blockDim.x) { sbelow[i] = 0u; sabove[i] = 0u; }
-    for (int i = threadIdx.x; i < K; i += blockDim.x) { scoff[i] = ws.cand_off[i]; scap[i] = ws.cap[i]; }
-    __syncthreads();
-
-    // this CTA's contiguous block of rows; thread t takes its elements t, t + NT, t + 2 NT, ... (row-major)
-    const long long per = (n + gridDim.x - 1) / gridDim.x;
-    const long long r0 = (long long)blockIdx.x * per;
-    const long long r1 = r0 + per < n ? r0 + per : n;
-    const int NT = blockDim.x;
-    long long row = r0 + threadIdx.x / D;
-    int d = threadIdx.x % D;
-    const int step_r = NT / D, step_d = NT % D;
-
-    auto handle = [&](int k, int dd, T x, long long rrow) {
-        if ((unsigned)k >= (unsigned)K) return;
-        const int kd = k * D + dd;
-        const T lo = spiv[2 * kd], hi = spiv[2 * kd + 1];
-        if (x < lo) {
-            red_shared_inc(&sbelow[kd]);
-        } else if (x > hi) {
-            // above the bracket: nothing to count (above = n_k - below - ties - listed)
-        } else if (lo == hi && x == lo) {
-            red_shared_inc(&sabove[kd]);  // the tie plateau (this array holds the tie counts)
-        } else {
-            // the closed bracket [lo, hi] and every NaN go to the list; with lo == hi (the sample saw a plateau
-            // of ties) the ties are counted, not listed
-            const unsigned rep = mn_rep((unsigned)rrow);  // by row, not by CTA: balanced for any row order
-            const unsigned pos = atomicAdd(&ws.ncand[(size_t)rep * KD + kd], 1u);
-            const unsigned cap = scap[k];
-            if (pos < cap) ws.cand[scoff[k] + ((size_t)rep * D + dd) * cap + pos] = x;
-        }
-    };
-
-    constexpr int U = 4;  // independent loads in flight per thread
-    while (row < r1) {
-        long long rr[U];
-        int dd[U], kk[U];
-        T xx[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            rr[u] = row;
-            dd[u] = d;
-            d += step_d;
-            row += step_r;
-            if (d >= D) { d -= D; ++row; }
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const bool ok = rr[u] < r1;
-            kk[u] = ok ? __ldg(code + rr[u]) : -1;
-            xx[u] = ok ? X[rr[u] * ldx + dd[u]] : (T)0;
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) handle(kk[u], dd[u], xx[u], rr[u]);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < KD; i += blockDim.x) {
-        const unsigned b = sbelow[i], a = sabove[i];
-        if (b) atomicAdd(&ws.below[i], b);
-        if (a) atomicAdd(&ws.above[i], a);
-    }
-}
-
-// The streaming pass, run form (any row stride or alignment): a CTA takes a chunk of <= 4096 consecutive rows,
-// counting-sorts the chunk's row ids by type in shared memory (codes only: 4 bytes per row), and its warps then
-// pull (type, 32-column group, 128-row segment) items: inside an item every row has the SAME type, so a lane keeps
-// the (lo, hi) pivots of its (type, dim) in registers and an element costs a shared-memory broadcast of the row id,
-// one address multiply-add, the load (a warp reads 32 consecutive elements of one row), two compares and a
-// predicated store -- about 10 instructions against 40-75 in the forms above, which look up the pivots per
-// element.  Bracket candidates collect in a lane-private shared-memory buffer and are appended to the (type, dim)
-// list once per item: ONE global atomic per lane and item instead of one per candidate.  The rows of a chunk are
-// read within microseconds of each other by one CTA, so the sectors two neighbouring rows share are fetched
-// from DRAM once (round 1 gathered rows in GLOBAL type order and paid 1.46x).
+// The streaming pass, run form (any alignment; rows less than 1 MiB apart): a CTA takes a chunk of <= 4096
+// consecutive rows, counting-sorts the chunk's row ids by type in shared memory (codes only: 4 bytes per row), and
+// its warps then pull (type, 32-column group, 128-row segment) items: inside an item every row has the SAME type, so
+// a lane keeps the (lo, hi) pivots of its (type, dim) in registers and an element costs a shared-memory broadcast of
+// the row id, one address multiply-add, the load (a warp reads 32 consecutive elements of one row), two compares and
+// a predicated store -- about 10 instructions against 40-75 in the earlier forms (history above), which looked up
+// the pivots per element.  Bracket candidates collect in a lane-private shared-memory buffer and are appended to the
+// (type, dim) list once per item: ONE global atomic per lane and item instead of one per candidate.  The rows of a
+// chunk are read within microseconds of each other by one CTA, so the sectors two neighbouring rows share are
+// fetched from DRAM once (round 1 gathered rows in GLOBAL type order and paid 1.46x).
 constexpr int MN_RUN_THREADS = 512;
 constexpr int MN_RUN_CMAX = 4096;      // rows per chunk: ids fit u16, <= 8 rows per thread in the sort
 constexpr int MN_RUN_SEG = 128;        // rows per item
+constexpr int MN_RUN_BUF = 128;        // bytes of a lane-private candidate buffer
+constexpr size_t MN_RUN_SMEM_MAX = 100 * 1024;  // two CTAs per SM
 template <typename T> struct MnRun {
-    static constexpr int B = 128 / (int)sizeof(T);  // lane-private candidate buffer entries (32 f32 / 16 f64)
+    static constexpr int B = MN_RUN_BUF / (int)sizeof(T);  // its entries (32 f32 / 16 f64)
     static constexpr int U = 32 / (int)sizeof(T);   // loads in flight per lane (8 / 4)
 };
 
@@ -929,8 +872,7 @@ __global__ void __launch_bounds__(MN_FIN_THREADS, 5)
 mn_finish_kernel(const T *__restrict__ X, long long n, int D, long long ldx, const int *__restrict__ code,
                  MnWs<T> ws, int STAGE, T *__restrict__ cent, double *__restrict__ cent64)
 {
-    using KO = KeyOf<T>;
-    using Key = typename KO::type;
+    using Key = typename KeyOf<T>::type;
     constexpr int BITS = sizeof(Key) * 8;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     T *s_stage = reinterpret_cast<T *>(smem_raw);
@@ -1071,21 +1013,8 @@ mn_finish_kernel(const T *__restrict__ X, long long n, int D, long long ldx, con
             if (g0 == 2 || g1 == 2) {
                 auto lst = [&](auto f) { lst_all([&](T x) { if (x == x) f(x); }); };
                 const long long s0 = g0 == 2 ? j0 : (g1 == 2 ? j1 : 0), s1 = g1 == 2 ? j1 : s0;  // s0 <= s1
-                bool done = false;
-                const bool finite = lo > -Inf<T>::pos() && hi < Inf<T>::pos();
-                // every orderable list element lies in [lo, hi]: linear bins over the bracket
-                if (finite && lo < hi) done = cta_select2_linear<T>(lst, s0, s1, lo, hi, lhist, lcoll, lsh, m0, m1);
-                if (!done) {
-                    // radix select; the digits above the first one in which key(lo) and key(hi) differ are common
-                    Key prefix = 0;
-                    int first = BITS - 8;
-                    if (finite) {
-                        const Key kl = KO::key(lo), kh = KO::key(hi);
-                        while (first > 0 && (kl >> first) == (kh >> first)) first -= 8;
-                        if (first < BITS - 8) prefix = (Key)((kl >> (first + 8)) << (first + 8));
-                    }
-                    cta_select2_raw<T>(lst, s0, s1, hist, sh, prefix, first, m0, m1);
-                }
+                // every orderable list element lies in the bracket [lo, hi]
+                cta_select2<T>(lst, s0, s1, lo, hi, lhist, lcoll, lsh, sh, m0, m1);
             }
             v0 = g0 == 1 ? lo : m0;
             v1 = g1 == 1 ? lo : m1;
@@ -1102,59 +1031,86 @@ mn_finish_kernel(const T *__restrict__ X, long long n, int D, long long ldx, con
 
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
-constexpr size_t MN_RUN_SMEM_MAX = 100 * 1024;  // two CTAs per SM
-template <typename T> static size_t mn_run_smem(int K, long long C)
-{
-    return (size_t)MnRun<T>::B * MN_RUN_THREADS * sizeof(T) + ((size_t)4 * K + 3 + C / MN_RUN_SEG + 1) * 4 + (size_t)C * 2 + 16;
-}
-
-static size_t mn_stream_smem(int K, int D, size_t elt)
-{
-    const size_t kd = (size_t)K * D;
-    return 2 * kd * elt + (size_t)K * 8 + 2 * kd * 4 + (size_t)K * 4;
-}
-
-template <typename T>
-static size_t mn_ws_bytes(long long n, int K, int D)
-{
-    const size_t kd = (size_t)K * D;
-    size_t b = 256;                                   // header
-    b += align256((size_t)K * 8);                     // type_cnt
-    b += align256((size_t)K * 4);                     // samp_cur
-    b += align256(kd * 4) * 2;                        // below, above
-    b += align256(kd * 4 * MN_REP);                   // ncand
-    b += align256((size_t)K * 8);                     // cand_off
-    b += align256((size_t)K * 4) * 3;                 // cap, sstride, scap
-    b += align256((size_t)K * 8);                     // samp_off
-    b += align256(kd * 2 * sizeof(T));                // piv
-    b += align256(((size_t)(n / 16) * 5 / 4 + (size_t)K * (MN_SAMPLE_MIN * 5 / 4 + 64 + 64)) * D * sizeof(T));  // samp
-    b += align256((size_t)(0.35 * (double)n * D) * sizeof(T) + (size_t)65 * MN_REP * kd * sizeof(T) + 4096);  // cand pool
-    return b;
-}
-
-template <typename T>
-static int median_run_stream(const T *X, long long n, int D, long long ldx, const int *code, int K, T *cent,
-                             double *cent64, void *workspace, cudaStream_t st)
-{
-    const size_t kd = (size_t)K * D;
+// the stream path's workspace (256-byte aligned regions)
+template <typename T> struct MnLayout {
     MnWs<T> ws;
-    unsigned char *p = (unsigned char *)workspace;
-    ws.hdr = (MnHeader *)p; p += 256;
-    ws.type_cnt = (unsigned long long *)p; p += align256((size_t)K * 8);
-    ws.samp_cur = (unsigned int *)p; p += align256((size_t)K * 4);
-    ws.below = (unsigned int *)p; p += align256(kd * 4);
-    ws.above = (unsigned int *)p; p += align256(kd * 4);
-    ws.ncand = (unsigned int *)p; p += align256(kd * 4 * MN_REP);
-    const size_t zero_bytes = (size_t)(p - (unsigned char *)workspace);
-    ws.cand_off = (unsigned long long *)p; p += align256((size_t)K * 8);
-    ws.cap = (unsigned int *)p; p += align256((size_t)K * 4);
-    ws.sstride = (unsigned int *)p; p += align256((size_t)K * 4);
-    ws.scap = (unsigned int *)p; p += align256((size_t)K * 4);
-    ws.samp_off = (unsigned long long *)p; p += align256((size_t)K * 8);
-    ws.piv = (T *)p; p += align256(kd * 2 * sizeof(T));
-    ws.samp = (T *)p; p += align256(((size_t)(n / 16) * 5 / 4 + (size_t)K * (MN_SAMPLE_MIN * 5 / 4 + 64 + 64)) * D * sizeof(T));
-    ws.cand = (T *)p;
-    PILOT_CUDA(cudaMemsetAsync(workspace, 0, zero_bytes, st));
+    size_t zero;   // the prefix zeroed at the start of every call: header and counters
+    size_t bytes;  // end of the last region
+};
+
+// carves the stream path's workspace at `base` (nullptr: only its size)
+template <typename T> static MnLayout<T> mn_workspace(void *base, long long n, int K, int D)
+{
+    const size_t kd = (size_t)K * D;
+    uintptr_t p = (uintptr_t)base;
+    const auto take = [&p](size_t bytes) { const uintptr_t r = p; p += align256(bytes); return r; };
+    MnLayout<T> l;
+    MnWs<T> &ws = l.ws;
+    ws.hdr = (MnHeader *)take(sizeof(MnHeader));
+    ws.type_cnt = (unsigned long long *)take((size_t)K * 8);
+    ws.samp_cur = (unsigned int *)take((size_t)K * 4);
+    ws.below = (unsigned int *)take(kd * 4);
+    ws.above = (unsigned int *)take(kd * 4);
+    ws.ncand = (unsigned int *)take(kd * 4 * MN_REP);
+    l.zero = p - (uintptr_t)base;
+    ws.cand_off = (unsigned long long *)take((size_t)K * 8);
+    ws.cap = (unsigned int *)take((size_t)K * 4);
+    ws.sstride = (unsigned int *)take((size_t)K * 4);
+    ws.scap = (unsigned int *)take((size_t)K * 4);
+    ws.samp_off = (unsigned long long *)take((size_t)K * 8);
+    ws.piv = (T *)take(kd * 2 * sizeof(T));
+    ws.samp = (T *)take(((size_t)(n / 16) * 5 / 4 + (size_t)K * (MN_SAMPLE_MIN * 5 / 4 + 64 + 64)) * D * sizeof(T));
+    ws.cand = (T *)take((size_t)(0.35 * (double)n * D) * sizeof(T) + (size_t)65 * MN_REP * kd * sizeof(T) + 4096);
+    l.bytes = p - (uintptr_t)base;
+    return l;
+}
+
+// which path computes the medians, and the run form's launch when it is the stream path
+struct MedianPath {
+    bool stream;        // the sampled-pivot stream path; otherwise the MSD radix select
+    long long ctas, C;  // the run form's CTAs and rows per chunk
+    size_t smem;        // its dynamic shared memory
+};
+
+// The stream path's limits on the shape alone, which is all the workspace query sees.  Its sample and list
+// workspace grows with K*D (f64: ~38 KB per (type, dim) plus 0.35 n D list elements, against 2 KB of histograms on
+// the radix path), so a large K*D takes the radix path.  The bound, 24 B per (type, dim) + 12 B per type within
+// 160 KiB, is the shared memory of an earlier form of the pass; it stays so that every input keeps its path.
+static bool mn_stream_shape_ok(long long n, int K, int D)
+{
+    return n >= 65536 && n < (1LL << 32) && K <= 4096 && 24 * (size_t)K * D + 12 * (size_t)K <= 160 * 1024;
+}
+
+// The stream path takes an input when its shape allows, its rows are less than 1 MiB apart (the run form's
+// chunk-relative byte offsets stay below 2^32) and the run form's shared memory holds its types.
+static MedianPath median_path(long long n, int K, int D, long long ldx, size_t elt)
+{
+    MedianPath p{};
+    if (!mn_stream_shape_ok(n, K, D) || ldx * (long long)elt >= (1LL << 20)) return p;
+    long long ctas = (n + 1023) / 1024;  // chunks of at least ~1024 rows
+    const long long cta_cap = (long long)sm_count() * 2;
+    if (ctas > cta_cap) ctas = cta_cap;
+    const long long m = (n + ctas * MN_RUN_CMAX - 1) / (ctas * MN_RUN_CMAX);  // chunks per CTA
+    long long C = (n + ctas * m - 1) / (ctas * m);
+    C = (C + 7) & ~7LL;
+    if (C > MN_RUN_CMAX) C = MN_RUN_CMAX;
+    const long long chunks = (n + C - 1) / C;
+    p.ctas = ctas < chunks ? ctas : chunks;
+    p.C = C;
+    // the kernel's dynamic shared memory: lane buffers, the sort's per-type tables, the item table, the row ids
+    p.smem = (size_t)MN_RUN_BUF * MN_RUN_THREADS + ((size_t)4 * K + 3 + C / MN_RUN_SEG + 1) * 4 + (size_t)C * 2 + 16;
+    p.stream = p.smem <= MN_RUN_SMEM_MAX;
+    return p;
+}
+
+template <typename T>
+static int median_run_stream(const T *X, long long n, int D, long long ldx, const int *code, int K,
+                             const MedianPath &path, T *cent, double *cent64, void *workspace, cudaStream_t st)
+{
+    const size_t kd = (size_t)K * D;
+    const MnLayout<T> l = mn_workspace<T>(workspace, n, K, D);
+    const MnWs<T> ws = l.ws;
+    PILOT_CUDA(cudaMemsetAsync(workspace, 0, l.zero, st));
     long long blocks = (n + 2047) / 2048;
     const long long cap = (long long)sm_count() * 8;
     if (blocks > cap) blocks = cap;
@@ -1173,41 +1129,9 @@ static int median_run_stream(const T *X, long long n, int D, long long ldx, cons
                                     (int)(MN_MCAP * sizeof(T))));
     mn_pivot_kernel<T><<<(unsigned)kd, 256, MN_MCAP * sizeof(T), st>>>(D, ws);
     PILOT_LAUNCH_CHECK();
-    bool streamed = false;
-    if (K <= 32768 && ldx * (long long)sizeof(T) < (1LL << 20)) {  // chunk-relative byte offsets stay below 2^32
-        // run form: chunk-sorted row ids, pivots in registers
-        const long long cta_cap = (long long)sm_count() * 2;
-        long long ctas = (n + 1023) / 1024;           // chunks of at least ~1024 rows
-        if (ctas > cta_cap) ctas = cta_cap;
-        const long long m = (n + ctas * MN_RUN_CMAX - 1) / (ctas * MN_RUN_CMAX);   // chunks per CTA
-        long long C = (n + ctas * m - 1) / (ctas * m);
-        C = (C + 7) & ~7LL;
-        if (C > MN_RUN_CMAX) C = MN_RUN_CMAX;
-        const size_t smem = mn_run_smem<T>(K, C);
-        if (smem <= MN_RUN_SMEM_MAX) {
-            PILOT_CUDA(cudaFuncSetAttribute(mn_stream_run_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const long long chunks = (n + C - 1) / C;
-            if (ctas > chunks) ctas = chunks;
-            mn_stream_run_kernel<T><<<(unsigned)ctas, MN_RUN_THREADS, smem, st>>>(X, n, D, ldx, code, K, (int)C, ws);
-            PILOT_LAUNCH_CHECK();
-            streamed = true;
-        }
-    }
-    if (!streamed) {
-        // element-thread form (huge row strides or type counts): pivots and counters of every (type, dim) in shared memory
-        const size_t smem = mn_stream_smem(K, D, sizeof(T));
-        int per_sm = 1;
-        PILOT_CUDA(cudaFuncSetAttribute(mn_stream_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        PILOT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mn_stream_kernel<T>, MN_THREADS, smem));
-        if (per_sm < 1) per_sm = 1;
-        if (per_sm > 4) per_sm = 4;
-        long long ctas = (long long)sm_count() * per_sm;
-        const long long need = (n * D + (long long)MN_THREADS * 16 - 1) / ((long long)MN_THREADS * 16);
-        if (ctas > need) ctas = need;
-        if (ctas < 1) ctas = 1;
-        mn_stream_kernel<T><<<(unsigned)ctas, MN_THREADS, smem, st>>>(X, n, D, ldx, code, K, ws);
-        PILOT_LAUNCH_CHECK();
-    }
+    PILOT_CUDA(cudaFuncSetAttribute(mn_stream_run_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)path.smem));
+    mn_stream_run_kernel<T><<<(unsigned)path.ctas, MN_RUN_THREADS, path.smem, st>>>(X, n, D, ldx, code, K, (int)path.C, ws);
+    PILOT_LAUNCH_CHECK();
     {
         // stage size from the expected list length: bracket fraction 5.5 / sqrt(sample) of an average type, + 25 %;
         // a longer list is selected from global memory instead (L2 resident), a shorter stage lets more CTAs share an SM
@@ -1226,16 +1150,12 @@ static int median_run_stream(const T *X, long long n, int D, long long ldx, cons
     return 0;
 }
 
-static bool median_use_sorted(long long n, int K, int D)
-{
-    return n >= 65536 && n < (1LL << 32) && K <= 4096 && mn_stream_smem(K, D, 8) <= MN_SMEM_MAX;
-}
-
 size_t median_ws_bytes(long long n, int K, int D)
 {
-    size_t a = median_ws_bytes_impl(K, D);
-    if (median_use_sorted(n, K, D)) {
-        const size_t b = mn_ws_bytes<double>(n, K, D);
+    // ldx and the dtype are unknown here: room for the f64 stream path whenever the shape allows it
+    size_t a = median_workspace(nullptr, K, D).bytes;
+    if (mn_stream_shape_ok(n, K, D)) {
+        const size_t b = mn_workspace<double>(nullptr, n, K, D).bytes;
         if (b > a) a = b;
     }
     return a;
@@ -1256,11 +1176,12 @@ extern "C" int pilot_centroid_median(const void *X, int dtype, int64_t n_cells, 
                     "pilot_centroid_median: workspace %zu < %zu bytes", workspace_bytes,
                     median_ws_bytes(n_cells, K, D));
     cudaStream_t st = (cudaStream_t)stream;
-    if (median_use_sorted(n_cells, K, D)) {
+    const MedianPath path = median_path(n_cells, K, D, ldx, dtype == PILOT_F32 ? sizeof(float) : sizeof(double));
+    if (path.stream) {
         if (dtype == PILOT_F32)
-            return median_run_stream<float>((const float *)X, n_cells, D, ldx, ct_code, K, (float *)centroids,
+            return median_run_stream<float>((const float *)X, n_cells, D, ldx, ct_code, K, path, (float *)centroids,
                                             centroids_f64, workspace, st);
-        return median_run_stream<double>((const double *)X, n_cells, D, ldx, ct_code, K, (double *)centroids,
+        return median_run_stream<double>((const double *)X, n_cells, D, ldx, ct_code, K, path, (double *)centroids,
                                          centroids_f64, workspace, st);
     }
     if (dtype == PILOT_F32)

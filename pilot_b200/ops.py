@@ -124,7 +124,7 @@ def median_fallbacks(K: int, D: int, device=None) -> int:
     the exact full-column fallback of the streaming path (reads the workspace; synchronises)."""
     device = device or torch.device("cuda", torch.cuda.current_device())
     ws = _workspace(1, device)
-    return int(ws[0:4].view(torch.int32).item())  # MsHeader.fail is the first word of the workspace
+    return int(ws[0:4].view(torch.int32).item())  # MnHeader.fail is the first word of the workspace
 
 
 def cdist(cent64: torch.Tensor, metric: str = "cosine") -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:

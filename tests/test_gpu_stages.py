@@ -114,24 +114,25 @@ def test_centroid_median_streaming_path(dtype, case):
 
 @pytest.mark.parametrize("dtype", [np.float32, np.float64])
 @pytest.mark.parametrize("n,K,D", [(70_001, 3, 50), (65_537, 64, 50), (100_003, 30, 33), (90_002, 5, 7), (66_001, 4, 1),
-                                   (80_003, 40, 128), (70_003, 2, 512), (70_001, 2, 600)])
-def test_centroid_median_column_form_shapes(dtype, n, K, D):
-    """The column-thread stream kernel (G x D thread grid, bulk-copied row tiles): row counts that leave a short,
-    16-byte-unaligned last tile, thread grids that do not fill their last warp, one CTA-wide column, D > 512
-    (vector form), and rows whose code is out of range (pandas' -1 for a missing label), which must be ignored."""
+                                   (80_003, 40, 128), (70_003, 2, 512), (70_001, 2, 600), (200_003, 3000, 1)])
+def test_centroid_median_run_form_shapes(dtype, n, K, D):
+    """The run form of the stream pass: row counts that leave a short last chunk, column groups narrower than 32
+    (several rows per step), D > 512, rows whose code is out of range (pandas' -1 for a missing label), which must be
+    ignored, and a base pointer that is not 16-byte aligned.  3000 types are more than the run form's shared memory
+    holds: that input takes the radix path."""
     rng = np.random.default_rng(n + D)
     X = rng.normal(size=(n, D)).astype(dtype)
     X[rng.integers(0, n, 300), rng.integers(0, D, 300)] = np.nan
     code = rng.integers(0, K, size=n).astype(np.int32)
     code[rng.integers(0, n, 500)] = -1
     code[rng.integers(0, n, 50)] = K + 3
-    code[-1] = K - 1            # the very last row (in the plain-store tail of the last tile) counts
+    code[-1] = K - 1            # the very last row (in the short last chunk) counts
     X[-1] = 1e6
     cent, cent64 = ops.centroid_median(dev(X), dev(code), K)
     want = np.stack([np.nanmedian(X[code == k], axis=0) for k in range(K)])
     np.testing.assert_array_equal(cent.cpu().numpy(), want.astype(dtype))
     np.testing.assert_array_equal(cent64.cpu().numpy(), want.astype(np.float64))
-    # a view that starts 4 bytes into an allocation: not 16-byte aligned -> the other stream kernels, same result
+    # a view that starts 4 bytes into an allocation, not 16-byte aligned: same result
     if D == 50:
         flat = torch.empty(n * D + 1, dtype=torch.from_numpy(X).dtype, device="cuda")
         Xo = flat[1:].view(n, D)
