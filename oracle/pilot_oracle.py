@@ -277,14 +277,15 @@ def sinkhorn2_np(a, b, M, reg, **kw):
     return float(np.sum(M * sinkhorn_stabilized_np(a, b, M, reg, **kw)))
 
 
-def sinkhorn2(a, b, M, reg, numItermax=1000, stopThr=1e-9, tau=1e3, return_info=False):
-    """C restatement (same statements as sinkhorn_stabilized_np)."""
+def sinkhorn2(a, b, M, reg, numItermax=1000, stopThr=1e-9, tau=1e3, return_info=False, check_every=20):
+    """C restatement (same statements as sinkhorn_stabilized_np).  check_every is POT's print_period: the
+    marginal error is evaluated when ii % check_every == 0."""
     a = np.ascontiguousarray(a, dtype=np.float64)
     b = np.ascontiguousarray(b, dtype=np.float64)
     M = np.ascontiguousarray(M, dtype=np.float64)
     info = _SkInfo()
     c = lib().pilot_oracle_sinkhorn2(M.shape[0], M.shape[1], _dp(a), _dp(b), _dp(M), float(reg),
-                                     int(numItermax), float(tau), float(stopThr), 20,
+                                     int(numItermax), float(tau), float(stopThr), int(check_every),
                                      ctypes.byref(info))
     if return_info:
         return float(c), dict(iters=info.iters, absorptions=info.absorptions,

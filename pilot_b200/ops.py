@@ -127,6 +127,16 @@ def median_fallbacks(K: int, D: int, device=None) -> int:
     return int(ws[0:4].view(torch.int32).item())  # MnHeader.fail is the first word of the workspace
 
 
+def sinkhorn_counters(device=None) -> dict:
+    """Diagnostic: the device counters of the LAST sinkhorn_pairs / sinkhorn_plans call on this stream (reads the
+    SkCounters header at the start of the workspace; synchronises).  n_redo: problems queued for the reference-form
+    kernel; n_tail: problems the DMMA panels handed to the warp-form tail kernel."""
+    device = device or torch.device("cuda", torch.cuda.current_device())
+    ws = _workspace(1, device)
+    fast, n_redo, slow, n_tail, tail = (int(x) for x in ws[0:40].view(torch.int64).tolist())
+    return dict(fast=fast, n_redo=n_redo, slow=slow, n_tail=n_tail, tail=tail)
+
+
 def cdist(cent64: torch.Tensor, metric: str = "cosine") -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """(cost[K,K], cost / cost.max(), cost.max()) for a scipy pdist metric name."""
     _require_cuda(cent64)
